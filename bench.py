@@ -25,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree may be read-only: importing the package from it leaves no __pycache__ there
 
 METRIC = "read_pairs_per_sec_matched"
 UNIT = "pairs/s"
@@ -50,6 +51,9 @@ def parse_args():
     ap.add_argument("--sweep-pairs", type=int, default=50_000_000)
     ap.add_argument("--total-pairs", type=int, default=100_000_000, help="config 3: pairs of the whole job, split over the ranks")
     ap.add_argument("--matcher-mbases", type=int, default=1024)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the match records of the timed path "
+                    "(main leg; --impl reference: the oracle's) as DIR/<gf_match field>.npy and their count as "
+                    "DIR/n_records.npy, float64, in (pair_idx, source) order")
     return ap.parse_args()
 
 
@@ -216,6 +220,25 @@ def gpu_records(torch, d_out, n):
     dt = match_dtype()
     raw = d_out[:n * dt.itemsize].cpu().numpy().view(dt)
     return np.sort(raw, order=["pair_idx", "source"])
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, recs):
+    """records (structured, match_dtype order) -> one float64 .npy per field + n_records.npy.  Beyond DUMP_BYTES a fixed,
+    seeded sample of the rows is written: the same rows whenever the record count is the same."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    fields = recs.dtype.names
+    rows = np.arange(len(recs))
+    cap = (DUMP_BYTES - 4096) // (8 * len(fields))      # (4096: the .npy headers)
+    if len(rows) > cap:
+        rows = np.sort(np.random.default_rng(0).choice(len(recs), cap, replace=False))
+    np.save(os.path.join(out_dir, "n_records.npy"), np.array([len(recs)], dtype=np.float64))
+    for f in fields:
+        np.save(os.path.join(out_dir, f + ".npy"), recs[f][rows].astype(np.float64))
+    log(f"dumped {len(rows)} of {len(recs)} records to {out_dir}")
 
 
 def parity_record(got, want, pairs, what):
@@ -411,8 +434,10 @@ def reference_arm(a, json_out, rank):
         oidx.scan(batch.slice(0, min(20000, batch.n)), threads=threads)
     t0 = time.perf_counter()
     for _ in range(a.steps):
-        oracle_scan_raw(oidx, batch, threads)
+        recs = oracle_scan_raw(oidx, batch, threads)
     dt = time.perf_counter() - t0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, recs)
     val = batch.n * a.steps / dt
     sample = (f"each step = the first {batch.n} pairs of the workload (bounded sample of its {a.pairs} pairs), "
               f"{a.steps} steps; C++ restatement of the Rust CPU path (oracle/), packs of 1000 pairs over all host threads")
@@ -457,6 +482,8 @@ def main():
     for x in legs:
         if x not in ALL_LEGS:
             raise SystemExit(f"unknown leg {x!r}")
+    if a.dump_outputs and "main" not in legs:
+        raise SystemExit("--dump-outputs writes the main leg's records: select the main leg")
     dev = torch.device("cuda", local_rank)
     threads = max(1, cpu_threads() // max(1, world))
     want_oracle = (not a.no_cpu_baseline) and world == 1
@@ -516,6 +543,8 @@ def main():
         matches_all = all_sum(n_matches)
         parity = None
         cpu = None
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, gpu_records(torch, d_outs[0], n_matches))
         if oracle is not None:
             got = gpu_records(torch, d_outs[0], n_matches)
             parity = parity_record(got, wl.oracle_all, P, f"all {P} pairs of the timed workload")
