@@ -1136,19 +1136,21 @@ int gf_adjust_fusion_break(gf_index* idx, const uint8_t* bytes, uint64_t n_bytes
     GF_CUDA_TRY(idx->ws_counters.reserve(sizeof(GfMapCounters)));
     cudaStream_t st = idx->stream;
     { int r = wait_prior_device_work(idx, st); if (r != GF_OK) return r; }
-    unsigned int* d_undef = &idx->ws_counters.as<GfMapCounters>()->n_ref_panic;
+    unsigned int* d_flagged = &idx->ws_counters.as<GfMapCounters>()->n_ref_panic;
     GF_CUDA_TRY(cudaMemsetAsync(idx->ws_counters.p, 0, sizeof(GfMapCounters), st));
     if (n_bytes) GF_CUDA_TRY(cudaMemcpyAsync(s.seq1.p, bytes, n_bytes, cudaMemcpyHostToDevice, st));
     GF_CUDA_TRY(cudaMemcpyAsync(s.off1.p, refs, sizeof(gf_break_ref) * (size_t)n_refs, cudaMemcpyHostToDevice, st));
     GF_CUDA_TRY(cudaMemcpyAsync(s.off2.p, jobs, sizeof(gf_break_job) * n_jobs, cudaMemcpyHostToDevice, st));
     int rc = gf_adjust_break_device(idx, s.seq1.as<uint8_t>(), s.off1.as<gf_break_ref>(), s.off2.as<gf_break_job>(), n_jobs,
-                                    s.out.as<gf_break_out>(), d_undef, st);
+                                    s.out.as<gf_break_out>(), d_flagged, st);
     if (rc != GF_OK) return rc;
     GF_CUDA_TRY(cudaMemcpyAsync(out, s.out.p, sizeof(gf_break_out) * n_jobs, cudaMemcpyDeviceToHost, st));
-    unsigned int n_undef = 0;
-    GF_CUDA_TRY(cudaMemcpyAsync(&n_undef, d_undef, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+    unsigned int n_flagged = 0;
+    GF_CUDA_TRY(cudaMemcpyAsync(&n_flagged, d_flagged, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
     GF_CUDA_TRY(cudaStreamSynchronize(st));
-    if (n_undef) return fail(GF_E_REF_PANIC, "a shifted break point lies outside its read (gf_break_out.status)");
+    if (n_flagged)
+        return fail(GF_E_REF_PANIC, "a shifted break point lies outside its read or a distance needs more than 640 columns "
+                                    "(gf_break_out.status)");
     return GF_OK;
 }
 

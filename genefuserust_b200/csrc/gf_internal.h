@@ -232,4 +232,4 @@ int gf_finish_records_device(gf_index* idx, const gf_match* d_in, const unsigned
                              cudaStream_t stream);
 int gf_fast_merge_device(gf_index* idx, const GfDevBatch& b, gf_merge_info* d_out, cudaStream_t stream);
 int gf_adjust_break_device(gf_index* idx, const uint8_t* d_bytes, const gf_break_ref* d_refs, const gf_break_job* d_jobs,
-                           uint64_t n_jobs, gf_break_out* d_out, unsigned int* d_n_undefined, cudaStream_t stream);
+                           uint64_t n_jobs, gf_break_out* d_out, unsigned int* d_n_flagged, cudaStream_t stream);

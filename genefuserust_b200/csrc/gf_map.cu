@@ -1315,7 +1315,7 @@ struct AdjustParams {
     const gf_break_job* jobs;
     unsigned long long n_jobs;
     gf_break_out* out;
-    unsigned int* n_undefined;
+    unsigned int* n_flagged;
 };
 __device__ __forceinline__ int ed_equal_len(const uint8_t* a, const uint8_t* b, int m) { /* both of length m */
     return m > 0 ? warp_edit_distance(a, m, false, b) : 0;
@@ -1331,16 +1331,19 @@ __global__ void __launch_bounds__(VF_WARPS * 32) k_adjust_break(AdjustParams P) 
         const uint8_t* rref = P.bytes + ref.right_off;
         const int len = (int)job.seq_len, nl = (int)ref.left_len, nr = (int)ref.right_len;
         int smallest = 0xFFFF, shift = 0, best_l = 0, best_r = 0;
-        bool undefined = false;
+        bool undefined = false, panic = false;
         for (int s = -3; s <= 3; s++) {
             const int left_len = job.read_break + s + 1, right_len = len - left_len;
             if (left_len < 0 || right_len < 0) { undefined = true; break; }
             const uint8_t* right_seq = seq + left_len;
+            /* calc_ed computes both full-length distances of every shift, winning or not, and the reference's edit_distance
+             * panics on more than 10 blocks (640 columns) on both sides; the two strings of each have equal length */
+            const int lc2 = min(left_len, nl), rc2 = min(right_len, nr);
+            if (lc2 > 640 || rc2 > 640) panic = true;
             /* the 20 bases on either side of the break decide (:340-372) */
-            const int lc = min(min(left_len, nl), 20), rc = min(min(right_len, nr), 20);
+            const int lc = min(lc2, 20), rc = min(rc2, 20);
             const int total = ed_equal_len(seq + left_len - lc, lref + nl - lc, lc) + ed_equal_len(right_seq, rref, rc);
             if (total < smallest) { /* strict: the first (most negative) best shift wins (:307-313) */
-                const int lc2 = min(left_len, nl), rc2 = min(right_len, nr);
                 best_l = ed_equal_len(seq + left_len - lc2, lref + nl - lc2, lc2);
                 best_r = ed_equal_len(right_seq, rref, rc2);
                 smallest = total;
@@ -1352,9 +1355,9 @@ __global__ void __launch_bounds__(VF_WARPS * 32) k_adjust_break(AdjustParams P) 
             o.shift = undefined ? 0 : shift;
             o.left_distance = undefined ? 0 : best_l;
             o.right_distance = undefined ? 0 : best_r;
-            o.status = undefined ? 1 : 0;
+            o.status = undefined ? 1 : panic ? 2 : 0; /* status 2 keeps the computed shift and distances */
             P.out[j] = o;
-            if (undefined) atomicAdd(P.n_undefined, 1u);
+            if (undefined || panic) atomicAdd(P.n_flagged, 1u);
         }
     }
 }
@@ -1649,10 +1652,11 @@ int gf_fast_merge_device(gf_index* idx, const GfDevBatch& b, gf_merge_info* d_ou
     return GF_OK;
 }
 
-/* report stage: adjust_fusion_break for n_jobs matches, everything already on the device; *d_n_undefined counts jobs whose
- * shifted break leaves the read */
+/* report stage: adjust_fusion_break for n_jobs matches, everything already on the device; *d_n_flagged counts jobs on which
+ * the reference would panic: a shifted break leaves the read (status 1) or a full-length distance needs more than 640
+ * columns (status 2) */
 int gf_adjust_break_device(gf_index* idx, const uint8_t* d_bytes, const gf_break_ref* d_refs, const gf_break_job* d_jobs,
-                           uint64_t n_jobs, gf_break_out* d_out, unsigned int* d_n_undefined, cudaStream_t st) {
+                           uint64_t n_jobs, gf_break_out* d_out, unsigned int* d_n_flagged, cudaStream_t st) {
     if (!n_jobs) return GF_OK;
     AdjustParams ap;
     ap.bytes = d_bytes;
@@ -1660,7 +1664,7 @@ int gf_adjust_break_device(gf_index* idx, const uint8_t* d_bytes, const gf_break
     ap.jobs = d_jobs;
     ap.n_jobs = n_jobs;
     ap.out = d_out;
-    ap.n_undefined = d_n_undefined;
+    ap.n_flagged = d_n_flagged;
     const uint64_t want = (n_jobs + VF_WARPS - 1) / VF_WARPS;
     const unsigned grid = (unsigned)std::min<uint64_t>(want, (uint64_t)idx->sm_count * resident_blocks(k_adjust_break, VF_WARPS * 32, 0));
     k_adjust_break<<<grid, VF_WARPS * 32, 0, st>>>(ap);

@@ -323,8 +323,10 @@ class FusionMapper:
     def adjust_fusion_break(self, results):
         """FusionResult::adjust_fusion_break (fusion_result.rs:299-397) for clustered matches.
         `results` = [(m_left_ref, m_right_ref, [(m_read.m_seq, m_read_break), ...]), ...] (bytes; the two reference strings
-        are what make_reference builds, :242-297).  Returns, per result, [(shift, m_left_distance, m_right_distance), ...];
-        the caller adds `shift` to m_read_break and to both gene positions (:317-319)."""
+        are what make_reference builds, :242-297).  Returns, per result, [(shift, m_left_distance, m_right_distance, status),
+        ...]; the caller adds `shift` to m_read_break and to both gene positions (:317-319).  status is gf_break_out.status:
+        1 = a shifted break leaves the read, 2 = a distance over more than 640 columns, where the reference panics; then
+        self.last_rc is GF_E_REF_PANIC."""
         arena = bytearray()
         refs = (gf_break_ref * max(1, len(results)))()
         jobs_l = []

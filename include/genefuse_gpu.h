@@ -289,7 +289,10 @@ typedef struct gf_break_out {
     int32_t left_distance;      /* new m_left_distance */
     int32_t right_distance;     /* new m_right_distance */
     int32_t status;             /* 0 ok; 1 = a shifted break lies outside the read (the reference's usize casts wrap there;
-                                   not reachable from make_match's breaks) — shift / distances are 0 and the call returns
+                                   not reachable from make_match's breaks) — shift / distances are 0; 2 = some shift's
+                                   full-length left or right comparison is longer than 640 columns, where the reference's
+                                   edit_distance panics (edit_distance.rs:94-100,177-196) — shift / distances are still the
+                                   exact ones.  1 takes precedence over 2.  Any job with status != 0 makes the call return
                                    GF_E_REF_PANIC */
 } gf_break_out;
 int gf_adjust_fusion_break(gf_index* idx, const uint8_t* bytes, uint64_t n_bytes, const gf_break_ref* refs, uint32_t n_refs,

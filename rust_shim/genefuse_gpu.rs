@@ -130,7 +130,9 @@ impl GpuIndex {
     /// FusionResult::adjust_fusion_break (src/core/fusion_result.rs:299-321) for every match of every result of one
     /// mapper: call it from cluster_matches right after fr.make_reference(..) (src/core/fusion_mapper.rs:438-456)
     /// instead of fr.adjust_fusion_break(); then for each match: m_read_break += shift, both positions += shift,
-    /// m_left_distance / m_right_distance = the returned distances.
+    /// m_left_distance / m_right_distance = the returned distances.  Where fr.adjust_fusion_break() would panic (a shifted
+    /// break outside the read, or a distance over more than 640 columns: gf_break_out.status 1 / 2) the call returns
+    /// GF_E_REF_PANIC and this Err(..).
     pub fn adjust_fusion_break(&self, arena: &[u8], refs: &[gf_break_ref], jobs: &[gf_break_job])
         -> Result<Vec<gf_break_out>, String> {
         let mut out = vec![gf_break_out::default(); jobs.len()];
