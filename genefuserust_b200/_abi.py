@@ -151,6 +151,13 @@ class gf_break_out(C.Structure):
     _fields_ = [("shift", C.c_int32), ("left_distance", C.c_int32), ("right_distance", C.c_int32), ("status", C.c_int32)]
 
 
+class gf_fastq_read_pair(C.Structure):
+    _fields_ = [("pair_idx", C.c_uint64), ("text_off", C.c_uint64), ("len", (C.c_uint32 * 4) * 2)]
+
+
+assert C.sizeof(gf_fastq_read_pair) == 48
+
+
 class gf_ref_contig(C.Structure):
     _fields_ = [("seq", C.c_void_p), ("len", C.c_uint64)]
 
@@ -180,7 +187,7 @@ EXPORTS = (
     "gf_index_set_output_mode",
     "gf_stream_create", "gf_stream_destroy", "gf_stream_push", "gf_stream_flush", "gf_stream_take", "gf_stream_get_counts",
     "gf_fastq_stream_create", "gf_fastq_stream_destroy", "gf_fastq_stream_feed", "gf_fastq_stream_finish",
-    "gf_fastq_stream_take", "gf_fastq_stream_get_counts",
+    "gf_fastq_stream_take", "gf_fastq_stream_get_counts", "gf_fastq_stream_keep_reads", "gf_fastq_stream_take_reads",
     "gf_pack_supported", "gf_pack_reads",
 )
 GF_FQ_PLAIN, GF_FQ_GZIP = 0, 1
@@ -277,6 +284,11 @@ def load_library():
     lib.gf_fastq_stream_take.restype = C.c_int
     lib.gf_fastq_stream_get_counts.argtypes = [C.c_void_p, P(C.c_uint64), P(C.c_uint64), P(C.c_uint64)]
     lib.gf_fastq_stream_get_counts.restype = C.c_int
+    lib.gf_fastq_stream_keep_reads.argtypes = [C.c_void_p]
+    lib.gf_fastq_stream_keep_reads.restype = C.c_int
+    lib.gf_fastq_stream_take_reads.argtypes = [C.c_void_p, P(gf_match), C.c_uint64, P(C.c_uint64), P(gf_fastq_read_pair), C.c_uint64,
+                                               P(C.c_uint64), C.c_void_p, C.c_uint64, P(C.c_uint64)]
+    lib.gf_fastq_stream_take_reads.restype = C.c_int
     lib.gf_index_set_output_mode.argtypes = [C.c_void_p, C.c_uint32]
     lib.gf_index_set_output_mode.restype = C.c_int
     lib.gf_reference_create.argtypes = [P(gf_ref_contig), C.c_uint32, C.c_int, P(C.c_void_p)]

@@ -122,6 +122,7 @@ void destroy_handle(gf_index* idx) {
     idx->ws_seq_lists.release();
     idx->fq[0].release();
     idx->fq[1].release();
+    idx->fq_reads.release();
     idx->bgzf_comp[0].release(); idx->bgzf_comp[1].release();
     idx->bgzf_members[0].release(); idx->bgzf_members[1].release();
     idx->bgzf_status.release();
@@ -925,13 +926,14 @@ int gf_fastq_fetch_text(gf_index* idx, int k, uint64_t from, uint64_t len, uint8
 
 int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t host1, const uint8_t* fq2, uint64_t host2, bool final_chunk,
                       gf_match* out, uint64_t out_cap, uint64_t* n_out, uint64_t* n_records, uint64_t consumed[2],
-                      const GfFastqMembers* members) {
+                      const GfFastqMembers* members, GfFastqReads* reads) {
     /* the text of a mate: host bytes, then (gf_fastq_stream, blocked gzip) the text of BGZF members that are still compressed */
     const uint64_t bytes1 = host1 + (members ? members[0].text_bytes : 0), bytes2 = host2 + (members && fq2 ? members[1].text_bytes : 0);
     if (!idx || !n_out || !n_records) return fail(GF_E_INVALID, "NULL argument");
     *n_out = 0;
     *n_records = 0;
     consumed[0] = consumed[1] = 0;
+    if (reads) { reads->pairs.clear(); reads->text.clear(); }
     if ((host1 && !fq1) || (host2 && !fq2)) return fail(GF_E_INVALID, "NULL FASTQ buffer");
     if (out_cap && !out) return fail(GF_E_INVALID, "out is NULL");
     std::lock_guard<std::mutex> lk(idx->mu);
@@ -1040,6 +1042,12 @@ int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t host1, const u
         GF_CUDA_TRY(cudaMemcpyAsync(&h->n_out2, sg.nout.as<unsigned long long>() + 1, sizeof(unsigned long long),
                                     cudaMemcpyDeviceToHost, st));
     }
+    if (reads) { /* the lines of the pairs behind the final records, while the text and its newline tables are resident */
+        const uint8_t* text[2] = {sg.seq1.as<uint8_t>(), pe ? sg.seq2.as<uint8_t>() : nullptr};
+        rc = gf_fastq_gather_reads(idx, text, n, mode ? sg.out2.as<gf_match>() : sg.out.as<gf_match>(),
+                                   sg.nout.as<unsigned long long>() + (mode ? 1 : 0), h, st);
+        if (rc != GF_OK) return rc;
+    }
     GF_CUDA_TRY(cudaMemcpyAsync(&h->counters, idx->ws_counters.p, sizeof(GfMapCounters), cudaMemcpyDeviceToHost, st));
     GF_CUDA_TRY(cudaMemcpyAsync(&h->n_out, sg.nout.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     GF_CUDA_TRY(cudaEventRecord(idx->ev_end, st));
@@ -1066,6 +1074,19 @@ int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t host1, const u
     } else {
         gf_sort_matches(out, n_rec);
     }
+    if (reads && n_rec) {
+        if ((unsigned long long)h->read_bytes != h->read_bytes64)
+            return fail(GF_E_LIMIT, "the lines of one chunk's matched pairs reach 2^32 bytes: feed smaller chunks");
+        rc = gf_fastq_regather_reads(idx, h->read_bytes64, st); /* (the arena was too small: grown, lines copied now) */
+        if (rc != GF_OK) return rc;
+        idx->stats.kernel_launches = idx->launches - launches0 + 3;
+        reads->pairs.resize(h->n_read_pairs);
+        reads->text.resize(h->read_bytes);
+        GF_CUDA_TRY(cudaMemcpy(reads->pairs.data(), idx->fq_reads.pairs.p, sizeof(gf_fastq_read_pair) * h->n_read_pairs,
+                               cudaMemcpyDeviceToHost));
+        if (h->read_bytes) GF_CUDA_TRY(cudaMemcpy(reads->text.data(), idx->fq_reads.text.p, h->read_bytes, cudaMemcpyDeviceToHost));
+        idx->stats.d2h_bytes += sizeof(gf_fastq_read_pair) * h->n_read_pairs + h->read_bytes + 2 * sizeof(uint32_t) + 8;
+    }
     if (h->counters.n_ref_panic)
         return fail(GF_E_REF_PANIC, "a candidate needs an edit distance over more than 640 columns (reference panics)");
     return GF_OK;
@@ -1073,7 +1094,8 @@ int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t host1, const u
 
 extern "C" {
 
-static_assert(sizeof(gf_map_stats) == 120 && sizeof(gf_match) == 48, "ABI layout (include/genefuse_gpu.h, _abi.py)");
+static_assert(sizeof(gf_map_stats) == 120 && sizeof(gf_match) == 48 && sizeof(gf_fastq_read_pair) == 48,
+              "ABI layout (include/genefuse_gpu.h, _abi.py)");
 int gf_get_map_stats(const gf_index* cidx, gf_map_stats* out) {
     gf_index* idx = const_cast<gf_index*>(cidx);
     if (!idx || !out) return fail(GF_E_INVALID, "NULL argument");

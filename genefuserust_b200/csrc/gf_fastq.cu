@@ -11,6 +11,8 @@
  *   k_nl_write   positions of all newlines, in order
  *   k_records    record i: sequence = (NL[4i], NL[4i+1]), quality = (NL[4i+2], NL[4i+3]); max length; checks
  */
+#include <algorithm>
+
 #include "gf_internal.h"
 #include "gf_inflate.cuh"
 
@@ -161,6 +163,142 @@ int gf_fastq_parse_device(const uint8_t* d_text, uint64_t bytes, GfFastqTable* o
             return GF_E_INVALID;
         }
     }
+    GF_CUDA_TRY(cudaGetLastError());
+    return GF_OK;
+}
+
+/* ---- the FASTQ lines of the pairs that have a record (gf_fastq_stream_keep_reads) ----
+ * Runs after k_verify / gf_finish_records_device, while the chunk's text and newline tables are still resident:
+ *   k_reads_mark     flag[local pair] = 1 for every record (the count is read on the device)
+ *   k_reads_size     per pair: the bytes of its 4 or 8 lines (0 when unflagged); 64-bit total beside it
+ *   two exclusive scans: flags -> slot in the ascending list of matched pairs, bytes -> offset in the text arena
+ *   k_reads_compact  descriptor of every matched pair at its slot
+ *   k_reads_gather   one warp per matched pair copies its lines, without the newlines, into the arena
+ * The arena holds the lines of the matched pairs only: it is not sized for the chunk's whole text (600 MB of device memory
+ * with the default 256 MiB chunks, for the ~1 MB that a chunk's matched pairs usually take).  Their total is known on the
+ * device only, so k_reads_gather is launched against the arena as it is and copies nothing when the total does not fit; the
+ * host sees that after the call's end-of-call synchronisation, grows the arena to the total and launches the gather again
+ * (gf_fastq_regather_reads): one extra launch and synchronisation each time the arena grows, which is rare — it is grow-only
+ * and starts at RD_ARENA_MIN. */
+namespace {
+
+constexpr int RD_THREADS = 256;
+constexpr size_t RD_ARENA_MIN = 256u << 10;
+
+__device__ __forceinline__ void line_span(const unsigned long long* __restrict__ nl, uint64_t j, unsigned long long* a,
+                                          uint32_t* len) {
+    /* line j spans (nl[j], nl[j + 1]) in the shifted table (nl[0] = -1: the +1 wraps to 0) */
+    *a = nl[j] + 1;
+    *len = (uint32_t)(nl[j + 1] - *a);
+}
+
+__global__ void k_reads_mark(const gf_match* __restrict__ rec, const unsigned long long* __restrict__ n_rec,
+                             uint32_t* __restrict__ flag) {
+    const unsigned long long n = *n_rec;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        flag[rec[i].pair_idx] = 1u;
+}
+
+__global__ void k_reads_size(const unsigned long long* __restrict__ nl1, const unsigned long long* __restrict__ nl2, uint64_t n,
+                             const uint32_t* __restrict__ flag, uint32_t* __restrict__ bytes,
+                             unsigned long long* __restrict__ total) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    unsigned long long b = 0;
+    if (flag[i]) {
+        /* record i = lines 4i .. 4i+3: its lines = from the name line's start to the quality line's end, less 3 newlines */
+        b = nl1[4 * i + 4] - (nl1[4 * i] + 1) - 3;
+        if (nl2) b += nl2[4 * i + 4] - (nl2[4 * i] + 1) - 3;
+        atomicAdd(total, b); /* 64-bit: the u32 scan of `bytes` must not wrap unnoticed (few pairs are flagged) */
+    }
+    bytes[i] = (uint32_t)b;
+}
+
+__global__ void k_reads_compact(const unsigned long long* __restrict__ nl1, const unsigned long long* __restrict__ nl2, uint64_t n,
+                                const uint32_t* __restrict__ flag, const uint32_t* __restrict__ slot,
+                                const uint32_t* __restrict__ off, gf_fastq_read_pair* __restrict__ out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || !flag[i]) return;
+    gf_fastq_read_pair p;
+    p.pair_idx = i;
+    p.text_off = off[i];
+    unsigned long long a;
+#pragma unroll
+    for (int l = 0; l < 4; l++) line_span(nl1, 4 * i + l, &a, &p.len[0][l]);
+#pragma unroll
+    for (int l = 0; l < 4; l++) {
+        p.len[1][l] = 0;
+        if (nl2) line_span(nl2, 4 * i + l, &a, &p.len[1][l]);
+    }
+    out[slot[i]] = p;
+}
+
+__global__ void k_reads_gather(const uint8_t* __restrict__ text1, const unsigned long long* __restrict__ nl1,
+                               const uint8_t* __restrict__ text2, const unsigned long long* __restrict__ nl2,
+                               const gf_fastq_read_pair* __restrict__ pairs, const uint32_t* __restrict__ n_pairs,
+                               const unsigned long long* __restrict__ total, uint64_t arena_cap, uint8_t* __restrict__ arena) {
+    const uint32_t lane = threadIdx.x & 31u;
+    if (*total > arena_cap) return; /* the host grows the arena and launches again */
+    const uint32_t n = *n_pairs;
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    for (uint64_t w = (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); w < n; w += warps) {
+        const uint64_t i = pairs[w].pair_idx;
+        uint8_t* dst = arena + pairs[w].text_off;
+        for (int m = 0; m < (nl2 ? 2 : 1); m++) {
+            const uint8_t* src = m ? text2 : text1;
+            const unsigned long long* nl = m ? nl2 : nl1;
+            for (int l = 0; l < 4; l++) {
+                unsigned long long a;
+                uint32_t len;
+                line_span(nl, 4 * i + l, &a, &len);
+                for (uint32_t b = lane; b < len; b += 32) dst[b] = __ldg(src + a + b);
+                dst += len;
+            }
+        }
+    }
+}
+
+}  // namespace
+
+int gf_fastq_gather_reads(gf_index* idx, const uint8_t* const text[2], uint64_t n, const gf_match* d_rec,
+                          const unsigned long long* d_n_rec, GfHostSlot* h, cudaStream_t st) {
+    GfFastqReadsWork& w = idx->fq_reads;
+    const bool pe = text[1] != nullptr;
+    const unsigned long long* nl1 = idx->fq[0].nl.as<unsigned long long>();
+    const unsigned long long* nl2 = pe ? idx->fq[1].nl.as<unsigned long long>() : nullptr;
+    w.text1 = text[0];
+    w.text2 = text[1];
+    w.n = n;
+    w.arena_used = 0;
+    if (n == 0) return GF_OK;
+    if (n >= 0xFFFFFFFFull) { gf_set_error("FASTQ chunk holds 2^32 or more records"); return GF_E_LIMIT; }
+    GF_CUDA_TRY(w.flag.reserve(sizeof(uint32_t) * (n + 1)));
+    GF_CUDA_TRY(w.slot.reserve(sizeof(uint32_t) * (n + 1)));
+    GF_CUDA_TRY(w.bytes.reserve(sizeof(uint32_t) * (n + 1)));
+    GF_CUDA_TRY(w.off.reserve(sizeof(uint32_t) * (n + 1)));
+    GF_CUDA_TRY(w.tmp.reserve(sizeof(uint32_t) * gf_scan_tmp_elems(n)));
+    GF_CUDA_TRY(w.total.reserve(sizeof(unsigned long long)));
+    GF_CUDA_TRY(w.pairs.reserve(sizeof(gf_fastq_read_pair) * n));
+    uint32_t *flag = w.flag.as<uint32_t>(), *slot = w.slot.as<uint32_t>(), *bytes = w.bytes.as<uint32_t>(), *off = w.off.as<uint32_t>();
+    unsigned long long* total = w.total.as<unsigned long long>();
+    GF_CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(uint32_t) * n, st));
+    GF_CUDA_TRY(cudaMemsetAsync(total, 0, sizeof(unsigned long long), st));
+    const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((n + RD_THREADS - 1) / RD_THREADS, 4ull * idx->sm_count));
+    const unsigned per_pair = (unsigned)((n + RD_THREADS - 1) / RD_THREADS);
+    k_reads_mark<<<grid, RD_THREADS, 0, st>>>(d_rec, d_n_rec, flag);
+    k_reads_size<<<per_pair, RD_THREADS, 0, st>>>(nl1, nl2, n, flag, bytes, total);
+    GF_CUDA_TRY(gf_exclusive_scan_u32(flag, slot, n, w.tmp.as<uint32_t>(), st));
+    GF_CUDA_TRY(gf_exclusive_scan_u32(bytes, off, n, w.tmp.as<uint32_t>(), st));
+    k_reads_compact<<<per_pair, RD_THREADS, 0, st>>>(nl1, nl2, n, flag, slot, off, w.pairs.as<gf_fastq_read_pair>());
+    GF_CUDA_TRY(w.text.reserve(RD_ARENA_MIN));
+    w.arena_used = w.text.cap;
+    k_reads_gather<<<grid, RD_THREADS, 0, st>>>(text[0], nl1, text[1], nl2, w.pairs.as<gf_fastq_read_pair>(), slot + n, total,
+                                                 w.arena_used, w.text.as<uint8_t>());
+    idx->launches += 4 + 2 * gf_scan_launches(n);
+    /* the totals travel with the call's other end-of-call copies into the pinned slot */
+    GF_CUDA_TRY(cudaMemcpyAsync(&h->n_read_pairs, slot + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    GF_CUDA_TRY(cudaMemcpyAsync(&h->read_bytes, off + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    GF_CUDA_TRY(cudaMemcpyAsync(&h->read_bytes64, total, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     GF_CUDA_TRY(cudaGetLastError());
     return GF_OK;
 }
@@ -392,5 +530,21 @@ int gf_bgzf_inflate_device(const uint8_t* d_comp, const GfBgzfMember* d_members,
     if (n == 0) return GF_OK;
     k_bgzf_inflate<<<(n + INF_WARPS - 1) / INF_WARPS, INF_WARPS * 32, INF_SMEM, st>>>(d_comp, d_members, n, d_text, d_status);
     GF_CUDA_TRY(cudaGetLastError());
+    return GF_OK;
+}
+
+int gf_fastq_regather_reads(gf_index* idx, uint64_t bytes, cudaStream_t st) {
+    GfFastqReadsWork& w = idx->fq_reads;
+    if (w.n == 0 || bytes <= w.arena_used) return GF_OK;
+    GF_CUDA_TRY(w.text.reserve(bytes));
+    w.arena_used = w.text.cap;
+    const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((w.n + RD_THREADS - 1) / RD_THREADS, 4ull * idx->sm_count));
+    const unsigned long long* nl2 = w.text2 ? idx->fq[1].nl.as<unsigned long long>() : nullptr;
+    k_reads_gather<<<grid, RD_THREADS, 0, st>>>(w.text1, idx->fq[0].nl.as<unsigned long long>(), w.text2, nl2,
+                                                 w.pairs.as<gf_fastq_read_pair>(), w.slot.as<uint32_t>() + w.n,
+                                                 w.total.as<unsigned long long>(), w.arena_used, w.text.as<uint8_t>());
+    idx->launches++;
+    GF_CUDA_TRY(cudaGetLastError());
+    GF_CUDA_TRY(cudaStreamSynchronize(st));
     return GF_OK;
 }

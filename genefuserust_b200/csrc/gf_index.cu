@@ -369,6 +369,11 @@ size_t gf_scan_tmp_elems(uint64_t n) { return scan_tmp_elems(n); }
 cudaError_t gf_exclusive_scan_u32(const uint32_t* in, uint32_t* out, uint64_t n, uint32_t* tmp, cudaStream_t st) {
     return exclusive_scan(in, out, n, tmp, st);
 }
+uint32_t gf_scan_launches(uint64_t n) {
+    if (n == 0) return 0;
+    const uint64_t nb = (n + SCAN_TILE - 1) / SCAN_TILE;
+    return 2 + (nb <= 1024 ? 1 : gf_scan_launches(nb));
+}
 
 /* ======================================================================================================= */
 namespace {

@@ -104,7 +104,11 @@ struct GfHostSlot { /* pinned host memory the device writes results of one call/
     GfMapCounters counters;
     unsigned long long n_out;
     unsigned long long n_out2; /* records left after the device-side filter (output mode != 0) */
-    unsigned long long pad[14];
+    /* gf_map_fastq_text with the reads kept: pairs that have a record, the bytes of their lines (32-bit scan) and the same
+     * bytes summed in 64 bits (they differ when a chunk's lines reach 2^32 bytes) */
+    unsigned int n_read_pairs, read_bytes;
+    unsigned long long read_bytes64;
+    unsigned long long pad[12];
 };
 
 /* gf_fastq.cu: FASTQ text already on the device -> per-record start/end/quality-start tables */
@@ -114,6 +118,23 @@ struct GfFastqTable {
     GfBuf nl, s, e, qs; /* newline positions; sequence start / end; quality start (u64 each) */
     GfBuf cnt, off, tmp; /* per-tile newline counts, their exclusive scan, scan workspace (kept between calls) */
     void release() { nl.release(); s.release(); e.release(); qs.release(); cnt.release(); off.release(); tmp.release(); }
+};
+
+/* gf_fastq.cu: device workspace of gf_fastq_gather_reads (grow-only) */
+struct GfFastqReadsWork {
+    GfBuf flag, slot, bytes, off, tmp, total; /* per local pair: record flag, its slot, its bytes, its text offset; scan workspace */
+    GfBuf pairs, text;                        /* descriptors of the matched pairs (48 B per pair of the chunk: their count is
+                                                 known on the device only); their lines back to back (grow-only, sized to the
+                                                 largest total seen) */
+    const uint8_t *text1 = nullptr, *text2 = nullptr; /* the last gather: the chunk's text, its pairs, the arena bytes it could use */
+    uint64_t n = 0, arena_used = 0;
+    void release() { flag.release(); slot.release(); bytes.release(); off.release(); tmp.release(); total.release(); pairs.release(); text.release(); }
+};
+/* gf_map_fastq_text's optional output: the lines of every pair that has a record, in ascending pair order (pair_idx counts
+ * from the start of the call's text, text_off into `text`) */
+struct GfFastqReads {
+    std::vector<gf_fastq_read_pair> pairs;
+    std::vector<uint8_t> text;
 };
 
 struct GfChunkEvents { /* start, after k_prep, k_seed, k_diag, the whole screen, exact + verify */
@@ -165,6 +186,7 @@ struct gf_index {
     /* mapping workspace (grow-only) */
     GfBuf ws_survivors, ws_counters, ws_gtbl;
     GfFastqTable fq[2];
+    GfFastqReadsWork fq_reads;
     GfBuf ws_seq_words, ws_seq_meta, ws_seq_seed, ws_seq_lists; /* split screen pipeline (gf_screen_split.cuh): sequence store
                                                                   (plane words, meta, seeds); counters + the two class lists */
     GfStage stage[GF_STAGES];
@@ -185,6 +207,7 @@ int gf_lookup_device(gf_index* idx, const uint32_t* kmers, uint64_t n, gf_lookup
 
 size_t gf_scan_tmp_elems(uint64_t n);
 cudaError_t gf_exclusive_scan_u32(const uint32_t* in, uint32_t* out, uint64_t n, uint32_t* tmp, cudaStream_t st);
+uint32_t gf_scan_launches(uint64_t n); /* kernels gf_exclusive_scan_u32 launches for n elements */
 
 /* final_chunk: the text ends the file (an unterminated last line is a line); otherwise it is ignored (streamed chunks) */
 int gf_fastq_parse_device(const uint8_t* d_text, uint64_t bytes, GfFastqTable* out, cudaStream_t st, bool final_chunk = true);
@@ -192,7 +215,16 @@ int gf_fastq_parse_device(const uint8_t* d_text, uint64_t bytes, GfFastqTable* o
  * returns how many bytes of buffer k they covered (the caller carries the rest over); pair_idx counts from 0. */
 int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t bytes1, const uint8_t* fq2, uint64_t bytes2, bool final_chunk,
                       gf_match* out, uint64_t out_cap, uint64_t* n_out, uint64_t* n_records, uint64_t consumed[2],
-                      const GfFastqMembers* members = nullptr /* [2]: BGZF members that follow the host text, inflated on the device */);
+                      const GfFastqMembers* members = nullptr /* [2]: BGZF members that follow the host text, inflated on the device */,
+                      GfFastqReads* reads = nullptr /* the lines of the pairs that have a record (nullptr: nothing is gathered) */);
+/* after the records of a FASTQ chunk are final (d_rec[0 .. *d_n_rec), local pair indices): gather the lines of every pair that
+ * has one from the chunk's text (text[1] = nullptr: single end) into idx->fq_reads, and queue the copies of the totals into h
+ * (n_read_pairs, read_bytes, read_bytes64).  n = records (pairs) of the chunk.  The lines are copied only when they fit the
+ * arena as it is: once the totals have arrived, gf_fastq_regather_reads(idx, h->read_bytes64, st) grows it and copies them
+ * when they did not (and returns at once when they did); the text and newline tables must still be resident. */
+int gf_fastq_gather_reads(gf_index* idx, const uint8_t* const text[2], uint64_t n, const gf_match* d_rec,
+                          const unsigned long long* d_n_rec, GfHostSlot* h, cudaStream_t st);
+int gf_fastq_regather_reads(gf_index* idx, uint64_t bytes, cudaStream_t st);
 /* after gf_map_fastq_text: bytes [from, from + len) of mate k's text as the device saw it (the unconsumed tail of a chunk) */
 int gf_fastq_fetch_text(gf_index* idx, int k, uint64_t from, uint64_t len, uint8_t* dst);
 

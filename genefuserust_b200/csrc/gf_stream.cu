@@ -241,6 +241,11 @@ struct gf_fastq_stream {
     double ms_bgzf = 0, ms_stream = 0, ms_map = 0; /* GF_DEBUG_TIMING: where the host time of the gzip path goes (mate 1's thread) */
     std::vector<gf_match> done, tmp;
     bool panic = false;
+    bool fed = false;
+    bool keep_reads = false;             /* gf_fastq_stream_keep_reads: the lines of the pairs behind `done` */
+    std::vector<gf_fastq_read_pair> reads; /* ascending pair_idx, text_off into read_text */
+    std::vector<uint8_t> read_text;
+    GfFastqReads chunk_reads;            /* what the last mapping call gathered */
     std::mutex mu;
     ~gf_fastq_stream() {
         for (int k = 0; k < 2; k++)
@@ -271,7 +276,7 @@ int fq_map_locked(gf_fastq_stream* s, bool final_chunk) {
     for (;;) {
         rc = gf_map_fastq_text(s->idx, s->text[0].p, s->text[0].fill, s->paired ? s->text[1].p : nullptr,
                                s->paired ? s->text[1].fill : 0, final_chunk, s->tmp.data(), s->tmp.size(), &got, &nrec, consumed,
-                               have_members ? mem : nullptr);
+                               have_members ? mem : nullptr, s->keep_reads ? &s->chunk_reads : nullptr);
         if (rc == GF_E_CAPACITY) { s->tmp.resize(got); continue; }
         break;
     }
@@ -282,6 +287,15 @@ int fq_map_locked(gf_fastq_stream* s, bool final_chunk) {
         gf_match m = s->tmp[i];
         m.pair_idx += s->records;
         s->done.push_back(m);
+    }
+    if (s->keep_reads) { /* pair numbers and text offsets of the chunk -> the stream's */
+        const uint64_t base = s->read_text.size();
+        for (gf_fastq_read_pair p : s->chunk_reads.pairs) {
+            p.pair_idx += s->records;
+            p.text_off += base;
+            s->reads.push_back(p);
+        }
+        s->read_text.insert(s->read_text.end(), s->chunk_reads.text.begin(), s->chunk_reads.text.end());
     }
     s->records += nrec;
     s->n_calls++;
@@ -598,6 +612,7 @@ int gf_fastq_stream_feed(gf_fastq_stream* s, const uint8_t* fq1, uint64_t n1, co
     if (!s->paired && n2) return sfail(GF_E_INVALID, "single-end stream fed with a second file");
     std::lock_guard<std::mutex> lk(s->mu);
     GF_CUDA_TRY(cudaSetDevice(s->idx->device));
+    s->fed = true;
     const uint8_t* in[2] = {fq1, fq2};
     uint64_t left[2] = {n1, n2};
     while (left[0] || left[1]) {
@@ -649,12 +664,47 @@ int gf_fastq_stream_finish(gf_fastq_stream* s) {
 int gf_fastq_stream_take(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out) {
     if (!s || !n_out) return sfail(GF_E_INVALID, "NULL argument");
     std::lock_guard<std::mutex> lk(s->mu);
+    if (s->keep_reads) return sfail(GF_E_INVALID, "the stream keeps reads: collect records with gf_fastq_stream_take_reads");
     *n_out = s->done.size();
     if (s->done.size() > out_cap) return sfail(GF_E_CAPACITY, "out_cap too small; *n_out holds the required count");
     if (!out && !s->done.empty()) return sfail(GF_E_INVALID, "out is NULL");
     sort_records(s->idx, s->done);
     if (!s->done.empty()) memcpy(out, s->done.data(), sizeof(gf_match) * s->done.size());
     s->done.clear();
+    if (s->panic) {
+        s->panic = false;
+        return sfail(GF_E_REF_PANIC, "a candidate needs an edit distance over more than 640 columns (reference panics)");
+    }
+    return GF_OK;
+}
+
+int gf_fastq_stream_keep_reads(gf_fastq_stream* s) {
+    if (!s) return sfail(GF_E_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lk(s->mu);
+    if (s->fed) return sfail(GF_E_INVALID, "gf_fastq_stream_keep_reads after the first feed");
+    s->keep_reads = true;
+    return GF_OK;
+}
+
+int gf_fastq_stream_take_reads(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out, gf_fastq_read_pair* pairs,
+                               uint64_t pairs_cap, uint64_t* n_pairs, uint8_t* text, uint64_t text_cap, uint64_t* n_text) {
+    if (!s || !n_out || !n_pairs || !n_text) return sfail(GF_E_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lk(s->mu);
+    if (!s->keep_reads) return sfail(GF_E_INVALID, "the stream does not keep reads (gf_fastq_stream_keep_reads)");
+    *n_out = s->done.size();
+    *n_pairs = s->reads.size();
+    *n_text = s->read_text.size();
+    if (s->done.size() > out_cap || s->reads.size() > pairs_cap || s->read_text.size() > text_cap)
+        return sfail(GF_E_CAPACITY, "a capacity is too small; *n_out, *n_pairs and *n_text hold the required counts");
+    if ((!out && !s->done.empty()) || (!pairs && !s->reads.empty()) || (!text && !s->read_text.empty()))
+        return sfail(GF_E_INVALID, "output buffer is NULL");
+    sort_records(s->idx, s->done);
+    if (!s->done.empty()) memcpy(out, s->done.data(), sizeof(gf_match) * s->done.size());
+    if (!s->reads.empty()) memcpy(pairs, s->reads.data(), sizeof(gf_fastq_read_pair) * s->reads.size());
+    if (!s->read_text.empty()) memcpy(text, s->read_text.data(), s->read_text.size());
+    s->done.clear();
+    s->reads.clear();
+    s->read_text.clear();
     if (s->panic) {
         s->panic = false;
         return sfail(GF_E_REF_PANIC, "a candidate needs an edit distance over more than 640 columns (reference panics)");

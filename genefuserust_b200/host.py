@@ -13,7 +13,7 @@ import os
 import numpy as np
 
 from ._abi import (GF_E_CAPACITY, GF_E_REF_PANIC, GF_OK, gf_alignable_result, gf_break_job, gf_break_out, gf_break_ref,
-                   gf_index_info, gf_lookup, gf_map_stats, gf_match, gf_merge_info, gf_gene_span, gf_params, gf_ref_contig,
+                   gf_fastq_read_pair, gf_index_info, gf_lookup, gf_map_stats, gf_match, gf_merge_info, gf_gene_span, gf_params, gf_ref_contig,
                    gf_reference_info, load_library)
 from .batch import ReadBatch
 
@@ -458,11 +458,15 @@ class FastqStream:
     """FastqReader / FastqReaderPair as a byte stream (gf_fastq_stream_*): feed raw file bytes (plain or gzip, pieces may end
     anywhere), whole records are split and mapped on the device; records are numbered from the start of the files."""
 
-    def __init__(self, mapper, paired=True, gz=False, chunk_bytes=0):
+    def __init__(self, mapper, paired=True, gz=False, chunk_bytes=0, keep_reads=False):
+        """keep_reads: gather the FASTQ lines of every pair that has a record on the device (collect them with take_reads)"""
         self.lib = mapper.lib
         h = C.c_void_p()
         _check(self.lib, self.lib.gf_fastq_stream_create(mapper.m_indexer.h, 1 if paired else 0, 1 if gz else 0, chunk_bytes, C.byref(h)))
         self.h = h
+        self.paired = paired
+        if keep_reads:
+            _check(self.lib, self.lib.gf_fastq_stream_keep_reads(self.h))
 
     def feed(self, fq1=b"", fq2=b""):
         _check(self.lib, self.lib.gf_fastq_stream_feed(self.h, fq1 if fq1 else None, len(fq1), fq2 if fq2 else None, len(fq2)))
@@ -481,6 +485,36 @@ class FastqStream:
                 continue
             _check(self.lib, rc, allow=(GF_E_REF_PANIC,))
             return [out[i] for i in range(n.value)]
+
+    def take_reads(self):
+        """(records, {pair_idx: ((name, seq, strand, qual) of mate 1, the same of mate 2 or None)}) of a stream that keeps
+        reads: the lines exactly as FastqReader::read yields them"""
+        caps = [4096, 4096, 1 << 20]
+        while True:
+            out = (gf_match * caps[0])()
+            pairs = (gf_fastq_read_pair * caps[1])()
+            text = (C.c_uint8 * caps[2])()
+            n, npair, ntext = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
+            rc = self.lib.gf_fastq_stream_take_reads(self.h, out, caps[0], C.byref(n), pairs, caps[1], C.byref(npair),
+                                                     text, caps[2], C.byref(ntext))
+            if rc == GF_E_CAPACITY:
+                caps = [max(caps[0], int(n.value)), max(caps[1], int(npair.value)), max(caps[2], int(ntext.value))]
+                continue
+            _check(self.lib, rc, allow=(GF_E_REF_PANIC,))
+            buf = bytes(text)[:ntext.value]
+            reads = {}
+            for i in range(npair.value):
+                p = pairs[i]
+                pos = p.text_off
+                mates = []
+                for m in range(2):
+                    lines = []
+                    for ln in p.len[m]:
+                        lines.append(buf[pos:pos + ln])
+                        pos += ln
+                    mates.append(tuple(lines))
+                reads[int(p.pair_idx)] = (mates[0], mates[1] if self.paired else None)
+            return [out[i] for i in range(n.value)], reads
 
     def counts(self):
         a, b, c = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)

@@ -403,6 +403,25 @@ int gf_fastq_stream_feed(gf_fastq_stream* s, const uint8_t* fq1, uint64_t n1, co
 int gf_fastq_stream_finish(gf_fastq_stream* s);
 int gf_fastq_stream_take(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out);
 int gf_fastq_stream_get_counts(const gf_fastq_stream* s, uint64_t* records, uint64_t* text_bytes, uint64_t* map_calls);
+/* Keeping the reads.  Everything after the scan needs the reads behind the records (ReadMatch::m_read and the original pair,
+ * sort_matches' name tie-break, adjust_fusion_break, the reports), and on the stream's path their text exists only on the
+ * device, only while its chunk is mapped.  gf_fastq_stream_keep_reads (before the first feed; GF_E_INVALID after it) makes the
+ * stream gather, per mapped chunk and on the device, the four lines of both mates of every pair that has a record, and copy
+ * them back with the records.  gf_fastq_stream_take_reads then returns what gf_fastq_stream_take would (same records, same
+ * order, same GF_E_REF_PANIC rule) plus one gf_fastq_read_pair per distinct pair_idx among them, in ascending pair_idx, and
+ * the text of their lines.  A capacity that is too small gives GF_E_CAPACITY with all three counts set and consumes nothing.
+ * On a stream that keeps reads gf_fastq_stream_take fails with GF_E_INVALID (reads are never dropped silently); on one that
+ * does not, gf_fastq_stream_take_reads does.  With GF_OUT_DROP_FILTERED only the pairs of surviving records come back. */
+typedef struct gf_fastq_read_pair {
+    uint64_t pair_idx;   /* as gf_match.pair_idx (counted from the start of the files) */
+    uint64_t text_off;   /* mate 1's four lines start here in the text buffer, back to back, then mate 2's */
+    uint32_t len[2][4];  /* [mate][name line, sequence, strand line, quality]; one trailing '\n' stripped, '\r' kept,
+                            exactly the lines FastqReader::read yields (gf_fastq.cu's rule); mate 2 all 0 for single end */
+} gf_fastq_read_pair;    /* 48 bytes */
+int gf_fastq_stream_keep_reads(gf_fastq_stream* s);
+int gf_fastq_stream_take_reads(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out,
+                               gf_fastq_read_pair* pairs, uint64_t pairs_cap, uint64_t* n_pairs,
+                               uint8_t* text, uint64_t text_cap, uint64_t* n_text);
 
 /* ---- the packed upload, as a host-side utility ----
  * With all four arenas of a batch in pinned host memory (and reads <= 256 bases) gf_map_pairs / gf_list_map_pairs do not copy

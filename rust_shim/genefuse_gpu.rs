@@ -62,6 +62,17 @@ extern "C" {
     fn gf_stream_flush(s: *mut gf_stream) -> c_int;
     fn gf_stream_take(s: *mut gf_stream, out: *mut gf_match, out_cap: u64, n_out: *mut u64) -> c_int;
     fn gf_stream_get_counts(s: *const gf_stream, pairs_pushed: *mut u64, map_calls: *mut u64) -> c_int;
+    fn gf_fastq_stream_create(idx: *mut gf_index, paired: c_int, format: c_int, chunk_bytes: u64,
+                              out: *mut *mut gf_fastq_stream) -> c_int;
+    fn gf_fastq_stream_destroy(s: *mut gf_fastq_stream);
+    fn gf_fastq_stream_feed(s: *mut gf_fastq_stream, fq1: *const u8, n1: u64, fq2: *const u8, n2: u64) -> c_int;
+    fn gf_fastq_stream_finish(s: *mut gf_fastq_stream) -> c_int;
+    fn gf_fastq_stream_take(s: *mut gf_fastq_stream, out: *mut gf_match, out_cap: u64, n_out: *mut u64) -> c_int;
+    fn gf_fastq_stream_get_counts(s: *const gf_fastq_stream, records: *mut u64, text_bytes: *mut u64, map_calls: *mut u64) -> c_int;
+    fn gf_fastq_stream_keep_reads(s: *mut gf_fastq_stream) -> c_int;
+    fn gf_fastq_stream_take_reads(s: *mut gf_fastq_stream, out: *mut gf_match, out_cap: u64, n_out: *mut u64,
+                                  pairs: *mut gf_fastq_read_pair, pairs_cap: u64, n_pairs: *mut u64,
+                                  text: *mut u8, text_cap: u64, n_text: *mut u64) -> c_int;
     fn gf_reference_create(contigs: *const gf_ref_contig, n_contigs: u32, device: c_int, out: *mut *mut gf_reference) -> c_int;
     fn gf_reference_destroy(r: *mut gf_reference);
     fn gf_alignable_filter(r: *mut gf_reference, seqs: *const u8, seq_off: *const u64, n_seqs: u64, alignable: *mut u8,
@@ -70,6 +81,12 @@ extern "C" {
 
 #[repr(C)] pub struct gf_stream { _private: [u8; 0] }
 #[repr(C)] pub struct gf_reference { _private: [u8; 0] }
+#[repr(C)] pub struct gf_fastq_stream { _private: [u8; 0] }
+/// include/genefuse_gpu.h: the FASTQ lines of one matched pair inside the text that gf_fastq_stream_take_reads returns
+#[repr(C)] #[derive(Clone, Copy, Default, Debug)]
+pub struct gf_fastq_read_pair { pub pair_idx: u64, pub text_off: u64, pub len: [[u32; 4]; 2] }
+pub const GF_FQ_PLAIN: c_int = 0;
+pub const GF_FQ_GZIP: c_int = 1;
 #[repr(C)] pub struct gf_ref_contig { pub seq: *const u8, pub len: u64 }
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)]
 pub struct gf_alignable_result {
@@ -201,6 +218,92 @@ impl PackStream {
     }
 }
 impl Drop for PackStream { fn drop(&mut self) { unsafe { gf_stream_destroy(self.s) } } }
+
+/// FastqReader / FastqReaderPair on raw file bytes (src/core/fastq_reader.rs:39-69,75-147,149-179): feed the files' bytes as
+/// they are read (`.fq` plain, `.fq.gz` with gzip = true: BGZF members are inflated on the device); whole records are split and
+/// mapped on the device.  With keep_reads the stream also returns the four lines of both mates of every matched pair, which is
+/// all a ReadMatch needs (take_reads); without it, take() returns the records alone.
+pub struct FastqStream { s: *mut gf_fastq_stream, paired: bool }
+unsafe impl Send for FastqStream {}
+unsafe impl Sync for FastqStream {} // calls on one stream are serialised inside the library
+
+/// (name, sequence, strand, quality) lines of one mate, as FastqReader::read yields them ('\n' stripped, '\r' kept)
+pub type FastqLines<'a> = (&'a [u8], &'a [u8], &'a [u8], &'a [u8]);
+
+/// what take_reads returns: the records and the lines of their pairs (ascending pair_idx)
+pub struct FastqReads { pub records: Vec<gf_match>, pub pairs: Vec<gf_fastq_read_pair>, pub text: Vec<u8>, paired: bool }
+impl FastqReads {
+    /// mate 1's and (paired) mate 2's lines of self.pairs[k]
+    pub fn lines(&self, k: usize) -> (FastqLines<'_>, Option<FastqLines<'_>>) {
+        let p = &self.pairs[k];
+        let mut pos = p.text_off as usize;
+        let mut mate = |m: usize| {
+            let mut l: [&[u8]; 4] = [&[]; 4];
+            for j in 0..4 { let n = p.len[m][j] as usize; l[j] = &self.text[pos..pos + n]; pos += n; }
+            (l[0], l[1], l[2], l[3])
+        };
+        let m1 = mate(0);
+        let m2 = if self.paired { Some(mate(1)) } else { None };
+        (m1, m2)
+    }
+    /// index into self.pairs of a record's pair
+    pub fn find(&self, pair_idx: u64) -> Option<usize> { self.pairs.binary_search_by_key(&pair_idx, |p| p.pair_idx).ok() }
+}
+
+impl FastqStream {
+    /// chunk_bytes = 0: 256 MiB of text per mate per mapping call
+    pub fn new(index: &GpuIndex, paired: bool, gzip: bool, chunk_bytes: u64, keep_reads: bool) -> Result<Self, String> {
+        let mut s: *mut gf_fastq_stream = std::ptr::null_mut();
+        let fmt = if gzip { GF_FQ_GZIP } else { GF_FQ_PLAIN };
+        if unsafe { gf_fastq_stream_create(index.h, paired as c_int, fmt, chunk_bytes, &mut s) } != 0 { return Err(last_error()); }
+        let st = Self { s, paired };
+        if keep_reads && unsafe { gf_fastq_stream_keep_reads(st.s) } != 0 { return Err(last_error()); }
+        Ok(st)
+    }
+    pub fn feed(&self, fq1: &[u8], fq2: &[u8]) -> Result<(), String> {
+        let rc = unsafe { gf_fastq_stream_feed(self.s, fq1.as_ptr(), fq1.len() as u64, fq2.as_ptr(), fq2.len() as u64) };
+        if rc != 0 { Err(last_error()) } else { Ok(()) }
+    }
+    /// end of the files: the last records are mapped
+    pub fn finish(&self) -> Result<(), String> { if unsafe { gf_fastq_stream_finish(self.s) } != 0 { Err(last_error()) } else { Ok(()) } }
+    pub fn take(&self) -> Result<Vec<gf_match>, String> {
+        let mut cap = 4096usize;
+        loop {
+            let mut out = vec![gf_match::default(); cap];
+            let mut n = 0u64;
+            let rc = unsafe { gf_fastq_stream_take(self.s, out.as_mut_ptr(), cap as u64, &mut n) };
+            if rc == GF_E_CAPACITY { cap = n as usize; continue; }
+            if rc != 0 { return Err(last_error()); }
+            out.truncate(n as usize);
+            return Ok(out);
+        }
+    }
+    /// the records (as take() would return them) and the lines of every pair among them
+    pub fn take_reads(&self) -> Result<FastqReads, String> {
+        let mut caps = [4096u64, 4096, 1 << 20];
+        loop {
+            let mut out = vec![gf_match::default(); caps[0] as usize];
+            let mut pairs = vec![gf_fastq_read_pair::default(); caps[1] as usize];
+            let mut text = vec![0u8; caps[2] as usize];
+            let mut n = [0u64; 3];
+            let rc = unsafe { gf_fastq_stream_take_reads(self.s, out.as_mut_ptr(), caps[0], &mut n[0], pairs.as_mut_ptr(), caps[1],
+                                                         &mut n[1], text.as_mut_ptr(), caps[2], &mut n[2]) };
+            if rc == GF_E_CAPACITY { for k in 0..3 { caps[k] = caps[k].max(n[k]); } continue; }
+            if rc != 0 { return Err(last_error()); } // GF_E_REF_PANIC included: the reference aborts there
+            out.truncate(n[0] as usize);
+            pairs.truncate(n[1] as usize);
+            text.truncate(n[2] as usize);
+            return Ok(FastqReads { records: out, pairs, text, paired: self.paired });
+        }
+    }
+    /// (records = pairs read so far, text bytes, mapping calls)
+    pub fn counts(&self) -> (u64, u64, u64) {
+        let (mut r, mut b, mut c) = (0u64, 0u64, 0u64);
+        unsafe { gf_fastq_stream_get_counts(self.s, &mut r, &mut b, &mut c) };
+        (r, b, c)
+    }
+}
+impl Drop for FastqStream { fn drop(&mut self) { unsafe { gf_fastq_stream_destroy(self.s) } } }
 
 /// The Matcher pass (src/core/fusion_mapper.rs:488-542, src/core/matcher.rs): the reference is scanned ONCE per FASTA.
 pub struct GpuReference { r: *mut gf_reference }
