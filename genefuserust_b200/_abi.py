@@ -188,6 +188,7 @@ EXPORTS = (
     "gf_stream_create", "gf_stream_destroy", "gf_stream_push", "gf_stream_flush", "gf_stream_take", "gf_stream_get_counts",
     "gf_fastq_stream_create", "gf_fastq_stream_destroy", "gf_fastq_stream_feed", "gf_fastq_stream_finish",
     "gf_fastq_stream_take", "gf_fastq_stream_get_counts", "gf_fastq_stream_keep_reads", "gf_fastq_stream_take_reads",
+    "gf_fastq_stream_create_list", "gf_fastq_stream_take_index", "gf_fastq_stream_take_reads_index",
     "gf_pack_supported", "gf_pack_reads",
 )
 GF_FQ_PLAIN, GF_FQ_GZIP = 0, 1
@@ -289,6 +290,14 @@ def load_library():
     lib.gf_fastq_stream_take_reads.argtypes = [C.c_void_p, P(gf_match), C.c_uint64, P(C.c_uint64), P(gf_fastq_read_pair), C.c_uint64,
                                                P(C.c_uint64), C.c_void_p, C.c_uint64, P(C.c_uint64)]
     lib.gf_fastq_stream_take_reads.restype = C.c_int
+    lib.gf_fastq_stream_create_list.argtypes = [P(C.c_void_p), C.c_uint32, C.c_int, C.c_int, C.c_uint64, P(C.c_void_p)]
+    lib.gf_fastq_stream_create_list.restype = C.c_int
+    lib.gf_fastq_stream_take_index.argtypes = [C.c_void_p, C.c_uint32, P(gf_match), C.c_uint64, P(C.c_uint64)]
+    lib.gf_fastq_stream_take_index.restype = C.c_int
+    lib.gf_fastq_stream_take_reads_index.argtypes = [C.c_void_p, C.c_uint32, P(gf_match), C.c_uint64, P(C.c_uint64),
+                                                     P(gf_fastq_read_pair), C.c_uint64, P(C.c_uint64), C.c_void_p, C.c_uint64,
+                                                     P(C.c_uint64)]
+    lib.gf_fastq_stream_take_reads_index.restype = C.c_int
     lib.gf_index_set_output_mode.argtypes = [C.c_void_p, C.c_uint32]
     lib.gf_index_set_output_mode.restype = C.c_int
     lib.gf_reference_create.argtypes = [P(gf_ref_contig), C.c_uint32, C.c_int, P(C.c_void_p)]

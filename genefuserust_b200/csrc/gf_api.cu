@@ -154,6 +154,26 @@ void destroy_handle(gf_index* idx) {
 
 }  // namespace
 
+/* list mode: all handles are locked in address order (two list calls sharing handles cannot deadlock) */
+struct ListLock {
+    std::vector<gf_index*> order;
+    explicit ListLock(gf_index* const* hs, uint32_t nh) : order(hs, hs + nh) {
+        std::sort(order.begin(), order.end());
+        for (gf_index* h : order) h->mu.lock();
+    }
+    ~ListLock() { for (auto it = order.rbegin(); it != order.rend(); ++it) (*it)->mu.unlock(); }
+};
+int gf_validate_list(gf_index* const* hs, uint32_t nh) {
+    if (!hs || nh == 0) return fail(GF_E_INVALID, "empty index list");
+    for (uint32_t h = 0; h < nh; h++) {
+        if (!hs[h]) return fail(GF_E_INVALID, "NULL index in the list");
+        if (hs[h]->device != hs[0]->device) return fail(GF_E_INVALID, "all indices of a list must live on one device");
+        for (uint32_t g = 0; g < h; g++)
+            if (hs[g] == hs[h]) return fail(GF_E_INVALID, "the same index is listed twice");
+    }
+    return GF_OK;
+}
+
 extern "C" {
 
 const char* gf_last_error(void) { return g_last_error.c_str(); }
@@ -783,30 +803,10 @@ int gf_map_pairs(gf_index* idx, const gf_batch* in, gf_match* out, uint64_t out_
     return map_host_batch(&idx, 1, in, &out, &out_cap, n_out);
 }
 
-/* list mode: all handles are locked in address order (two list calls sharing handles cannot deadlock) */
-struct ListLock {
-    std::vector<gf_index*> order;
-    explicit ListLock(gf_index* const* hs, uint32_t nh) : order(hs, hs + nh) {
-        std::sort(order.begin(), order.end());
-        for (gf_index* h : order) h->mu.lock();
-    }
-    ~ListLock() { for (auto it = order.rbegin(); it != order.rend(); ++it) (*it)->mu.unlock(); }
-};
-static int validate_list(gf_index* const* hs, uint32_t nh) {
-    if (!hs || nh == 0) return fail(GF_E_INVALID, "empty index list");
-    for (uint32_t h = 0; h < nh; h++) {
-        if (!hs[h]) return fail(GF_E_INVALID, "NULL index in the list");
-        if (hs[h]->device != hs[0]->device) return fail(GF_E_INVALID, "all indices of a list must live on one device");
-        for (uint32_t g = 0; g < h; g++)
-            if (hs[g] == hs[h]) return fail(GF_E_INVALID, "the same index is listed twice");
-    }
-    return GF_OK;
-}
-
 int gf_list_map_pairs(gf_index* const* idx, uint32_t n_idx, const gf_batch* in, gf_match* const* out, const uint64_t* out_cap,
                       uint64_t* n_out) {
     if (!n_out || !out_cap || !out) return fail(GF_E_INVALID, "NULL argument");
-    int rc = validate_list(idx, n_idx);
+    int rc = gf_validate_list(idx, n_idx);
     if (rc != GF_OK) return rc;
     rc = validate_batch(in);
     if (rc != GF_OK) return rc;
@@ -819,7 +819,7 @@ int gf_list_map_pairs(gf_index* const* idx, uint32_t n_idx, const gf_batch* in, 
 int gf_map_pairs_device_list(gf_index* const* idx, uint32_t n_idx, const gf_batch* in_dev, gf_match* const* d_out,
                              uint64_t out_cap, uint64_t* const* d_n_out, void* cuda_stream) {
     if (!d_out || !d_n_out) return fail(GF_E_INVALID, "NULL argument");
-    int rc = validate_list(idx, n_idx);
+    int rc = gf_validate_list(idx, n_idx);
     if (rc != GF_OK) return rc;
     rc = validate_batch(in_dev);
     if (rc != GF_OK) return rc;
@@ -908,43 +908,43 @@ int gf_map_pairs_device(gf_index* idx, const gf_batch* in_dev, gf_match* d_out, 
 
 int gf_map_fastq(gf_index* idx, const uint8_t* fq1, uint64_t bytes1, const uint8_t* fq2, uint64_t bytes2, gf_match* out,
                  uint64_t out_cap, uint64_t* n_out, uint64_t* n_records) {
+    if (!idx) return fail(GF_E_INVALID, "NULL argument");
     uint64_t consumed[2];
-    return gf_map_fastq_text(idx, fq1, bytes1, fq2, bytes2, true, out, out_cap, n_out, n_records, consumed);
+    return gf_map_fastq_text(&idx, 1, fq1, bytes1, fq2, bytes2, true, &out, &out_cap, n_out, n_records, consumed);
 }
 
 } /* extern "C" */
 
-int gf_fastq_fetch_text(gf_index* idx, int k, uint64_t from, uint64_t len, uint8_t* dst) {
-    if (!idx || (len && !dst)) return fail(GF_E_INVALID, "NULL argument");
-    std::lock_guard<std::mutex> lk(idx->mu);
-    GF_CUDA_TRY(cudaSetDevice(idx->device));
-    const GfBuf& b = k ? idx->stage[0].seq2 : idx->stage[0].seq1;
-    if (from + len > b.cap) return fail(GF_E_INVALID, "text range outside the staged chunk");
-    if (len) GF_CUDA_TRY(cudaMemcpy(dst, b.as<uint8_t>() + from, len, cudaMemcpyDeviceToHost));
-    return GF_OK;
-}
-
-int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t host1, const uint8_t* fq2, uint64_t host2, bool final_chunk,
-                      gf_match* out, uint64_t out_cap, uint64_t* n_out, uint64_t* n_records, uint64_t consumed[2],
-                      const GfFastqMembers* members, GfFastqReads* reads) {
+int gf_map_fastq_text(gf_index* const* hs, uint32_t nh, const uint8_t* fq1, uint64_t host1, const uint8_t* fq2, uint64_t host2,
+                      bool final_chunk, gf_match* const* out, const uint64_t* out_cap, uint64_t* n_out, uint64_t* n_records,
+                      uint64_t consumed[2], const GfFastqMembers* members, GfFastqReads* reads, bool* panic,
+                      std::vector<uint8_t>* tail) {
     /* the text of a mate: host bytes, then (gf_fastq_stream, blocked gzip) the text of BGZF members that are still compressed */
     const uint64_t bytes1 = host1 + (members ? members[0].text_bytes : 0), bytes2 = host2 + (members && fq2 ? members[1].text_bytes : 0);
-    if (!idx || !n_out || !n_records) return fail(GF_E_INVALID, "NULL argument");
-    *n_out = 0;
+    if (!hs || !nh || !hs[0] || !n_out || !n_records) return fail(GF_E_INVALID, "NULL argument");
     *n_records = 0;
     consumed[0] = consumed[1] = 0;
-    if (reads) { reads->pairs.clear(); reads->text.clear(); }
+    for (uint32_t h = 0; h < nh; h++) {
+        n_out[h] = 0;
+        if (panic) panic[h] = false;
+        if (reads) { reads[h].pairs.clear(); reads[h].text.clear(); }
+    }
     if ((host1 && !fq1) || (host2 && !fq2)) return fail(GF_E_INVALID, "NULL FASTQ buffer");
-    if (out_cap && !out) return fail(GF_E_INVALID, "out is NULL");
-    std::lock_guard<std::mutex> lk(idx->mu);
+    for (uint32_t h = 0; h < nh; h++)
+        if (out_cap[h] && !out[h]) return fail(GF_E_INVALID, "out is NULL");
+    ListLock lk(hs, nh);
+    gf_index* idx = hs[0]; /* the text, its newline tables, the sequence store and the gathered lines live in idx's workspace */
     GF_CUDA_TRY(cudaSetDevice(idx->device));
-    idx->stats = gf_map_stats{};
-    idx->stats_pending = false;
     const bool pe = fq2 != nullptr;
     cudaStream_t st = idx->stream;
     GfStage& sg = idx->stage[0];
-    { int r = wait_prior_device_work(idx, st); if (r != GF_OK) return r; }
-    GF_CUDA_TRY(cudaEventRecord(idx->ev_start, st));
+    for (uint32_t h = 0; h < nh; h++) {
+        hs[h]->stats = gf_map_stats{};
+        hs[h]->stats_pending = false;
+        int r = wait_prior_device_work(hs[h], st);
+        if (r != GF_OK) return r;
+        GF_CUDA_TRY(cudaEventRecord(hs[h]->ev_start, st));
+    }
     /* raw text -> device (the sequence and quality "arenas" are the text itself) */
     GF_CUDA_TRY(sg.seq1.reserve(bytes1 + 32));
     if (host1) GF_CUDA_TRY(cudaMemcpyAsync(sg.seq1.p, fq1, host1, cudaMemcpyHostToDevice, st));
@@ -995,19 +995,30 @@ int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t host1, const u
     int rc = gf_fastq_parse_device(sg.seq1.as<uint8_t>(), bytes1, &idx->fq[0], st, final_chunk);
     if (rc == GF_OK && pe) rc = gf_fastq_parse_device(sg.seq2.as<uint8_t>(), bytes2, &idx->fq[1], st, final_chunk);
     if (rc != GF_OK) return rc;
-    GF_CUDA_TRY(cudaEventRecord(idx->ev_ingest, st)); /* end of the ingest (the parse synchronises on its record count) */
+    for (uint32_t h = 0; h < nh; h++) /* end of the ingest (the parse synchronises on its record count) */
+        GF_CUDA_TRY(cudaEventRecord(hs[h]->ev_ingest, st));
     const uint64_t n = pe ? std::min(idx->fq[0].n_records, idx->fq[1].n_records) : idx->fq[0].n_records;
     *n_records = n;
-    idx->stats.n_pairs = n;
+    for (uint32_t h = 0; h < nh; h++) hs[h]->stats.n_pairs = n;
     idx->stats.h2d_bytes = host1 + (pe ? host2 : 0) + h2d_members;
-    if (n == 0) return GF_OK;
     /* bytes the n whole records cover = one past the newline that ends record n - 1's quality line (shifted table: nl[4 n]) */
-    for (int k = 0; k < (pe ? 2 : 1); k++) {
+    for (int k = 0; k < (pe ? 2 : 1) && n; k++) {
         unsigned long long end = 0;
         GF_CUDA_TRY(cudaMemcpyAsync(&end, idx->fq[k].nl.as<unsigned long long>() + 4 * n, sizeof(end), cudaMemcpyDeviceToHost, st));
         GF_CUDA_TRY(cudaStreamSynchronize(st));
         consumed[k] = std::min<uint64_t>(end + 1, k ? bytes2 : bytes1);
     }
+    /* the unconsumed text of a mate whose members were inflated here exists on the device only: it goes back now, before any
+     * other call on idx can reuse the staging buffer */
+    for (int k = 0; k < (pe ? 2 : 1) && tail && members && !final_chunk; k++) {
+        tail[k].clear();
+        if (!members[k].n_members) continue;
+        const uint64_t from = consumed[k], len = (k ? bytes2 : bytes1) - from;
+        tail[k].resize(len);
+        if (len) GF_CUDA_TRY(cudaMemcpyAsync(tail[k].data(), (k ? sg.seq2 : sg.seq1).as<uint8_t>() + from, len, cudaMemcpyDeviceToHost, st));
+        GF_CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    if (n == 0) return GF_OK;
     GfDevBatch db{};
     db.n = n;
     db.seq1 = db.qual1 = sg.seq1.as<uint8_t>();
@@ -1026,68 +1037,120 @@ int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t host1, const u
     }
     if (db.max_len == 0) db.max_len = 1;
     const uint64_t cap = (pe ? 2 : 1) * n;
-    GF_CUDA_TRY(sg.out.reserve(sizeof(gf_match) * cap));
-    GF_CUDA_TRY(sg.nout.reserve(2 * sizeof(unsigned long long)));
-    const unsigned long long launches0 = idx->launches;
-    rc = gf_map_device_batch(idx, db, sg.out.as<gf_match>(), cap, sg.nout.as<unsigned long long>(), st, nullptr, true);
-    if (rc != GF_OK) return rc;
-    GfHostSlot* h = &idx->h_slots[0];
-    const uint32_t mode = idx->out_mode;
-    if (mode) {
-        GF_CUDA_TRY(sg.out2.reserve(sizeof(gf_match) * cap));
-        GF_CUDA_TRY(sg.keys.reserve(sizeof(unsigned long long) * cap));
-        rc = gf_finish_records_device(idx, sg.out.as<gf_match>(), sg.nout.as<unsigned long long>(), cap, sg.out2.as<gf_match>(),
-                                      sg.keys.as<unsigned long long>(), sg.nout.as<unsigned long long>() + 1, mode, st);
+    std::vector<unsigned long long> launches0(nh);
+    for (uint32_t h = 0; h < nh; h++) launches0[h] = hs[h]->launches;
+    GfRecordLists lists{};
+    for (uint32_t h = 0; h < nh; h++) { /* every index into its own record buffers; k_prep ran once, for hs[0] */
+        gf_index* x = hs[h];
+        GfStage& xs = x->stage[0];
+        GF_CUDA_TRY(xs.out.reserve(sizeof(gf_match) * cap));
+        GF_CUDA_TRY(xs.nout.reserve(2 * sizeof(unsigned long long)));
+        rc = gf_map_device_batch(x, db, xs.out.as<gf_match>(), cap, xs.nout.as<unsigned long long>(), st, nullptr, true,
+                                 h ? idx : nullptr);
         if (rc != GF_OK) return rc;
-        GF_CUDA_TRY(cudaMemcpyAsync(&h->n_out2, sg.nout.as<unsigned long long>() + 1, sizeof(unsigned long long),
-                                    cudaMemcpyDeviceToHost, st));
+        const uint32_t mode = x->out_mode;
+        if (mode) {
+            GF_CUDA_TRY(xs.out2.reserve(sizeof(gf_match) * cap));
+            GF_CUDA_TRY(xs.keys.reserve(sizeof(unsigned long long) * cap));
+            rc = gf_finish_records_device(x, xs.out.as<gf_match>(), xs.nout.as<unsigned long long>(), cap, xs.out2.as<gf_match>(),
+                                          xs.keys.as<unsigned long long>(), xs.nout.as<unsigned long long>() + 1, mode, st);
+            if (rc != GF_OK) return rc;
+            GF_CUDA_TRY(cudaMemcpyAsync(&x->h_slots[0].n_out2, xs.nout.as<unsigned long long>() + 1, sizeof(unsigned long long),
+                                        cudaMemcpyDeviceToHost, st));
+        }
+        if (h < GF_FASTQ_LIST_MAX) {
+            lists.rec[h] = mode ? xs.out2.as<gf_match>() : xs.out.as<gf_match>();
+            lists.n[h] = xs.nout.as<unsigned long long>() + (mode ? 1 : 0);
+        }
     }
+    GfHostSlot* h0 = &idx->h_slots[0];
     if (reads) { /* the lines of the pairs behind the final records, while the text and its newline tables are resident */
+        if (nh > GF_FASTQ_LIST_MAX) return fail(GF_E_LIMIT, "more than 64 indices keep reads in one mapping call");
         const uint8_t* text[2] = {sg.seq1.as<uint8_t>(), pe ? sg.seq2.as<uint8_t>() : nullptr};
-        rc = gf_fastq_gather_reads(idx, text, n, mode ? sg.out2.as<gf_match>() : sg.out.as<gf_match>(),
-                                   sg.nout.as<unsigned long long>() + (mode ? 1 : 0), h, st);
+        rc = gf_fastq_gather_reads(idx, text, n, lists, nh, h0, st);
         if (rc != GF_OK) return rc;
     }
-    GF_CUDA_TRY(cudaMemcpyAsync(&h->counters, idx->ws_counters.p, sizeof(GfMapCounters), cudaMemcpyDeviceToHost, st));
-    GF_CUDA_TRY(cudaMemcpyAsync(&h->n_out, sg.nout.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    GF_CUDA_TRY(cudaEventRecord(idx->ev_end, st));
-    GF_CUDA_TRY(cudaEventSynchronize(idx->ev_end));
-    idx->busy = false;
-    rc = check_flags(*h);
-    if (rc != GF_OK) return rc;
-    accumulate(idx->stats, *h);
-    float ms = 0;
-    GF_CUDA_TRY(cudaEventElapsedTime(&ms, idx->ev_start, idx->ev_end));
-    idx->stats.ms_total = ms;
-    GF_CUDA_TRY(cudaEventElapsedTime(&idx->stats.ms_ingest, idx->ev_start, idx->ev_ingest));
-    idx->stats.kernel_launches = idx->launches - launches0 + 3;
-    const uint64_t n_rec = mode ? h->n_out2 : h->n_out;
-    *n_out = n_rec;
-    if (n_rec > out_cap) return fail(GF_E_CAPACITY, "out_cap too small; *n_out holds the required count");
-    if (n_rec) GF_CUDA_TRY(cudaMemcpy(out, mode ? sg.out2.p : sg.out.p, sizeof(gf_match) * n_rec, cudaMemcpyDeviceToHost));
-    idx->stats.d2h_bytes = sizeof(gf_match) * n_rec + sizeof(GfMapCounters) + 8;
-    if (mode & GF_OUT_BUCKET_ORDER) {
-        std::vector<unsigned long long> keys(n_rec);
-        if (n_rec) GF_CUDA_TRY(cudaMemcpy(keys.data(), sg.keys.p, sizeof(unsigned long long) * n_rec, cudaMemcpyDeviceToHost));
-        idx->stats.d2h_bytes += sizeof(unsigned long long) * n_rec;
-        order_by_keys(out, keys, n_rec);
-    } else {
-        gf_sort_matches(out, n_rec);
+    for (uint32_t h = 0; h < nh; h++) {
+        gf_index* x = hs[h];
+        GF_CUDA_TRY(cudaMemcpyAsync(&x->h_slots[0].counters, x->ws_counters.p, sizeof(GfMapCounters), cudaMemcpyDeviceToHost, st));
+        GF_CUDA_TRY(cudaMemcpyAsync(&x->h_slots[0].n_out, x->stage[0].nout.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        GF_CUDA_TRY(cudaEventRecord(x->ev_end, st));
     }
-    if (reads && n_rec) {
-        if ((unsigned long long)h->read_bytes != h->read_bytes64)
+    GF_CUDA_TRY(cudaEventSynchronize(hs[nh - 1]->ev_end));
+    bool too_small = false;
+    for (uint32_t h = 0; h < nh; h++) {
+        gf_index* x = hs[h];
+        const GfHostSlot& hx = x->h_slots[0];
+        x->busy = false;
+        rc = check_flags(hx);
+        if (rc != GF_OK) return rc;
+        accumulate(x->stats, hx);
+        float ms = 0;
+        GF_CUDA_TRY(cudaEventElapsedTime(&ms, x->ev_start, x->ev_end));
+        x->stats.ms_total = ms;
+        GF_CUDA_TRY(cudaEventElapsedTime(&x->stats.ms_ingest, x->ev_start, x->ev_ingest));
+        x->stats.kernel_launches = x->launches - launches0[h] + (h ? 0 : 3);
+        n_out[h] = x->out_mode ? hx.n_out2 : hx.n_out;
+        too_small |= n_out[h] > out_cap[h];
+    }
+    if (too_small) return fail(GF_E_CAPACITY, "out_cap too small; *n_out holds the required count");
+    bool any_panic = false, any_rec = false;
+    for (uint32_t h = 0; h < nh; h++) {
+        gf_index* x = hs[h];
+        const uint32_t mode = x->out_mode;
+        const uint64_t n_rec = n_out[h];
+        gf_match* o = out[h];
+        if (n_rec) GF_CUDA_TRY(cudaMemcpy(o, mode ? x->stage[0].out2.p : x->stage[0].out.p, sizeof(gf_match) * n_rec, cudaMemcpyDeviceToHost));
+        x->stats.d2h_bytes = sizeof(gf_match) * n_rec + sizeof(GfMapCounters) + 8;
+        if (mode & GF_OUT_BUCKET_ORDER) {
+            std::vector<unsigned long long> keys(n_rec);
+            if (n_rec) GF_CUDA_TRY(cudaMemcpy(keys.data(), x->stage[0].keys.p, sizeof(unsigned long long) * n_rec, cudaMemcpyDeviceToHost));
+            x->stats.d2h_bytes += sizeof(unsigned long long) * n_rec;
+            order_by_keys(o, keys, n_rec);
+        } else {
+            gf_sort_matches(o, n_rec);
+        }
+        any_rec |= n_rec != 0;
+        const bool p = x->h_slots[0].counters.n_ref_panic != 0;
+        any_panic |= p;
+        if (panic) panic[h] = p;
+    }
+    if (reads && any_rec) {
+        if ((unsigned long long)h0->read_bytes != h0->read_bytes64)
             return fail(GF_E_LIMIT, "the lines of one chunk's matched pairs reach 2^32 bytes: feed smaller chunks");
-        rc = gf_fastq_regather_reads(idx, h->read_bytes64, st); /* (the arena was too small: grown, lines copied now) */
+        rc = gf_fastq_regather_reads(idx, h0->read_bytes64, st); /* (the arena was too small: grown, lines copied now) */
         if (rc != GF_OK) return rc;
-        idx->stats.kernel_launches = idx->launches - launches0 + 3;
-        reads->pairs.resize(h->n_read_pairs);
-        reads->text.resize(h->read_bytes);
-        GF_CUDA_TRY(cudaMemcpy(reads->pairs.data(), idx->fq_reads.pairs.p, sizeof(gf_fastq_read_pair) * h->n_read_pairs,
+        idx->stats.kernel_launches = idx->launches - launches0[0] + 3;
+        /* the union of the indices' pairs; one index: it is that index's list as it is (every mask is 1) */
+        GfFastqReads uni;
+        GfFastqReads& u = nh == 1 ? reads[0] : uni;
+        u.pairs.resize(h0->n_read_pairs);
+        u.text.resize(h0->read_bytes);
+        GF_CUDA_TRY(cudaMemcpy(u.pairs.data(), idx->fq_reads.pairs.p, sizeof(gf_fastq_read_pair) * h0->n_read_pairs,
                                cudaMemcpyDeviceToHost));
-        if (h->read_bytes) GF_CUDA_TRY(cudaMemcpy(reads->text.data(), idx->fq_reads.text.p, h->read_bytes, cudaMemcpyDeviceToHost));
-        idx->stats.d2h_bytes += sizeof(gf_fastq_read_pair) * h->n_read_pairs + h->read_bytes + 2 * sizeof(uint32_t) + 8;
+        if (h0->read_bytes) GF_CUDA_TRY(cudaMemcpy(u.text.data(), idx->fq_reads.text.p, h0->read_bytes, cudaMemcpyDeviceToHost));
+        idx->stats.d2h_bytes += sizeof(gf_fastq_read_pair) * h0->n_read_pairs + h0->read_bytes + 2 * sizeof(uint32_t) + 8;
+        if (nh > 1) { /* each index gets its own pairs, its text laid out as a stream over that index alone lays it out */
+            std::vector<unsigned long long> masks(h0->n_read_pairs);
+            GF_CUDA_TRY(cudaMemcpy(masks.data(), idx->fq_reads.pair_mask.p, sizeof(unsigned long long) * masks.size(),
+                                   cudaMemcpyDeviceToHost));
+            idx->stats.d2h_bytes += sizeof(unsigned long long) * masks.size();
+            for (size_t j = 0; j < masks.size(); j++) {
+                const gf_fastq_read_pair& p = u.pairs[j];
+                uint64_t len = 0;
+                for (int m = 0; m < 2; m++)
+                    for (int l = 0; l < 4; l++) len += p.len[m][l];
+                for (uint32_t h = 0; h < nh; h++) {
+                    if (!((masks[j] >> h) & 1ull)) continue;
+                    gf_fastq_read_pair q = p;
+                    q.text_off = reads[h].text.size();
+                    reads[h].pairs.push_back(q);
+                    reads[h].text.insert(reads[h].text.end(), u.text.begin() + p.text_off, u.text.begin() + p.text_off + len);
+                }
+            }
+        }
     }
-    if (h->counters.n_ref_panic)
+    if (any_panic)
         return fail(GF_E_REF_PANIC, "a candidate needs an edit distance over more than 640 columns (reference panics)");
     return GF_OK;
 }

@@ -169,17 +169,18 @@ int gf_fastq_parse_device(const uint8_t* d_text, uint64_t bytes, GfFastqTable* o
 
 /* ---- the FASTQ lines of the pairs that have a record (gf_fastq_stream_keep_reads) ----
  * Runs after k_verify / gf_finish_records_device, while the chunk's text and newline tables are still resident:
- *   k_reads_mark     flag[local pair] = 1 for every record (the count is read on the device)
- *   k_reads_size     per pair: the bytes of its 4 or 8 lines (0 when unflagged); 64-bit total beside it
- *   two exclusive scans: flags -> slot in the ascending list of matched pairs, bytes -> offset in the text arena
- *   k_reads_compact  descriptor of every matched pair at its slot
+ *   k_reads_mark     bit h of mask[local pair] for every record of index h of the list (the counts are read on the device)
+ *   k_reads_size     per pair: a 0/1 "has a record" word and the bytes of its 4 or 8 lines (0 when unmarked); 64-bit total
+ *   two exclusive scans: the 0/1 words -> slot in the ascending list of matched pairs, bytes -> offset in the text arena
+ *   k_reads_compact  descriptor and mask of every matched pair at its slot
  *   k_reads_gather   one warp per matched pair copies its lines, without the newlines, into the arena
  * The arena holds the lines of the matched pairs only: it is not sized for the chunk's whole text (600 MB of device memory
  * with the default 256 MiB chunks, for the ~1 MB that a chunk's matched pairs usually take).  Their total is known on the
  * device only, so k_reads_gather is launched against the arena as it is and copies nothing when the total does not fit; the
  * host sees that after the call's end-of-call synchronisation, grows the arena to the total and launches the gather again
  * (gf_fastq_regather_reads): one extra launch and synchronisation each time the arena grows, which is rare — it is grow-only
- * and starts at RD_ARENA_MIN. */
+ * and starts at RD_ARENA_MIN.  A list stream gathers the union of its indices' matched pairs once; the masks tell the host
+ * which index each pair belongs to. */
 namespace {
 
 constexpr int RD_THREADS = 256;
@@ -192,20 +193,24 @@ __device__ __forceinline__ void line_span(const unsigned long long* __restrict__
     *len = (uint32_t)(nl[j + 1] - *a);
 }
 
-__global__ void k_reads_mark(const gf_match* __restrict__ rec, const unsigned long long* __restrict__ n_rec,
-                             uint32_t* __restrict__ flag) {
-    const unsigned long long n = *n_rec;
+/* blockIdx.y = index h of the list */
+__global__ void k_reads_mark(GfRecordLists lists, unsigned long long* __restrict__ mask) {
+    const uint32_t h = blockIdx.y;
+    const gf_match* __restrict__ rec = lists.rec[h];
+    const unsigned long long n = *lists.n[h];
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
-        flag[rec[i].pair_idx] = 1u;
+        atomicOr(&mask[rec[i].pair_idx], 1ull << h);
 }
 
 __global__ void k_reads_size(const unsigned long long* __restrict__ nl1, const unsigned long long* __restrict__ nl2, uint64_t n,
-                             const uint32_t* __restrict__ flag, uint32_t* __restrict__ bytes,
+                             const unsigned long long* __restrict__ mask, uint32_t* __restrict__ has, uint32_t* __restrict__ bytes,
                              unsigned long long* __restrict__ total) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     unsigned long long b = 0;
-    if (flag[i]) {
+    const bool marked = mask[i] != 0;
+    has[i] = marked ? 1u : 0u; /* (the scan counts pairs, not mask bits) */
+    if (marked) {
         /* record i = lines 4i .. 4i+3: its lines = from the name line's start to the quality line's end, less 3 newlines */
         b = nl1[4 * i + 4] - (nl1[4 * i] + 1) - 3;
         if (nl2) b += nl2[4 * i + 4] - (nl2[4 * i] + 1) - 3;
@@ -215,10 +220,13 @@ __global__ void k_reads_size(const unsigned long long* __restrict__ nl1, const u
 }
 
 __global__ void k_reads_compact(const unsigned long long* __restrict__ nl1, const unsigned long long* __restrict__ nl2, uint64_t n,
-                                const uint32_t* __restrict__ flag, const uint32_t* __restrict__ slot,
-                                const uint32_t* __restrict__ off, gf_fastq_read_pair* __restrict__ out) {
+                                const unsigned long long* __restrict__ mask, const uint32_t* __restrict__ slot,
+                                const uint32_t* __restrict__ off, gf_fastq_read_pair* __restrict__ out,
+                                unsigned long long* __restrict__ out_mask) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || !flag[i]) return;
+    if (i >= n) return;
+    const unsigned long long mk = mask[i];
+    if (!mk) return;
     gf_fastq_read_pair p;
     p.pair_idx = i;
     p.text_off = off[i];
@@ -231,6 +239,7 @@ __global__ void k_reads_compact(const unsigned long long* __restrict__ nl1, cons
         if (nl2) line_span(nl2, 4 * i + l, &a, &p.len[1][l]);
     }
     out[slot[i]] = p;
+    out_mask[slot[i]] = mk;
 }
 
 __global__ void k_reads_gather(const uint8_t* __restrict__ text1, const unsigned long long* __restrict__ nl1,
@@ -260,8 +269,8 @@ __global__ void k_reads_gather(const uint8_t* __restrict__ text1, const unsigned
 
 }  // namespace
 
-int gf_fastq_gather_reads(gf_index* idx, const uint8_t* const text[2], uint64_t n, const gf_match* d_rec,
-                          const unsigned long long* d_n_rec, GfHostSlot* h, cudaStream_t st) {
+int gf_fastq_gather_reads(gf_index* idx, const uint8_t* const text[2], uint64_t n, const GfRecordLists& lists, uint32_t nh,
+                          GfHostSlot* h, cudaStream_t st) {
     GfFastqReadsWork& w = idx->fq_reads;
     const bool pe = text[1] != nullptr;
     const unsigned long long* nl1 = idx->fq[0].nl.as<unsigned long long>();
@@ -272,24 +281,28 @@ int gf_fastq_gather_reads(gf_index* idx, const uint8_t* const text[2], uint64_t 
     w.arena_used = 0;
     if (n == 0) return GF_OK;
     if (n >= 0xFFFFFFFFull) { gf_set_error("FASTQ chunk holds 2^32 or more records"); return GF_E_LIMIT; }
-    GF_CUDA_TRY(w.flag.reserve(sizeof(uint32_t) * (n + 1)));
+    GF_CUDA_TRY(w.mask.reserve(sizeof(unsigned long long) * n));
+    GF_CUDA_TRY(w.has.reserve(sizeof(uint32_t) * (n + 1)));
     GF_CUDA_TRY(w.slot.reserve(sizeof(uint32_t) * (n + 1)));
     GF_CUDA_TRY(w.bytes.reserve(sizeof(uint32_t) * (n + 1)));
     GF_CUDA_TRY(w.off.reserve(sizeof(uint32_t) * (n + 1)));
     GF_CUDA_TRY(w.tmp.reserve(sizeof(uint32_t) * gf_scan_tmp_elems(n)));
     GF_CUDA_TRY(w.total.reserve(sizeof(unsigned long long)));
     GF_CUDA_TRY(w.pairs.reserve(sizeof(gf_fastq_read_pair) * n));
-    uint32_t *flag = w.flag.as<uint32_t>(), *slot = w.slot.as<uint32_t>(), *bytes = w.bytes.as<uint32_t>(), *off = w.off.as<uint32_t>();
+    GF_CUDA_TRY(w.pair_mask.reserve(sizeof(unsigned long long) * n));
+    unsigned long long* mask = w.mask.as<unsigned long long>();
+    uint32_t *has = w.has.as<uint32_t>(), *slot = w.slot.as<uint32_t>(), *bytes = w.bytes.as<uint32_t>(), *off = w.off.as<uint32_t>();
     unsigned long long* total = w.total.as<unsigned long long>();
-    GF_CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(uint32_t) * n, st));
+    GF_CUDA_TRY(cudaMemsetAsync(mask, 0, sizeof(unsigned long long) * n, st));
     GF_CUDA_TRY(cudaMemsetAsync(total, 0, sizeof(unsigned long long), st));
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((n + RD_THREADS - 1) / RD_THREADS, 4ull * idx->sm_count));
     const unsigned per_pair = (unsigned)((n + RD_THREADS - 1) / RD_THREADS);
-    k_reads_mark<<<grid, RD_THREADS, 0, st>>>(d_rec, d_n_rec, flag);
-    k_reads_size<<<per_pair, RD_THREADS, 0, st>>>(nl1, nl2, n, flag, bytes, total);
-    GF_CUDA_TRY(gf_exclusive_scan_u32(flag, slot, n, w.tmp.as<uint32_t>(), st));
+    k_reads_mark<<<dim3(grid, nh), RD_THREADS, 0, st>>>(lists, mask);
+    k_reads_size<<<per_pair, RD_THREADS, 0, st>>>(nl1, nl2, n, mask, has, bytes, total);
+    GF_CUDA_TRY(gf_exclusive_scan_u32(has, slot, n, w.tmp.as<uint32_t>(), st));
     GF_CUDA_TRY(gf_exclusive_scan_u32(bytes, off, n, w.tmp.as<uint32_t>(), st));
-    k_reads_compact<<<per_pair, RD_THREADS, 0, st>>>(nl1, nl2, n, flag, slot, off, w.pairs.as<gf_fastq_read_pair>());
+    k_reads_compact<<<per_pair, RD_THREADS, 0, st>>>(nl1, nl2, n, mask, slot, off, w.pairs.as<gf_fastq_read_pair>(),
+                                                      w.pair_mask.as<unsigned long long>());
     GF_CUDA_TRY(w.text.reserve(RD_ARENA_MIN));
     w.arena_used = w.text.cap;
     k_reads_gather<<<grid, RD_THREADS, 0, st>>>(text[0], nl1, text[1], nl2, w.pairs.as<gf_fastq_read_pair>(), slot + n, total,

@@ -122,19 +122,30 @@ struct GfFastqTable {
 
 /* gf_fastq.cu: device workspace of gf_fastq_gather_reads (grow-only) */
 struct GfFastqReadsWork {
-    GfBuf flag, slot, bytes, off, tmp, total; /* per local pair: record flag, its slot, its bytes, its text offset; scan workspace */
-    GfBuf pairs, text;                        /* descriptors of the matched pairs (48 B per pair of the chunk: their count is
-                                                 known on the device only); their lines back to back (grow-only, sized to the
-                                                 largest total seen) */
+    GfBuf mask, has, slot, bytes, off, tmp, total; /* per local pair: bit h = index h of the list has a record of it, 0/1 "has a
+                                                      record", its slot, its bytes, its text offset; scan workspace */
+    GfBuf pairs, pair_mask, text;             /* descriptors of the matched pairs and their masks (per pair of the chunk: their
+                                                 count is known on the device only); their lines back to back (grow-only, sized
+                                                 to the largest total seen) */
     const uint8_t *text1 = nullptr, *text2 = nullptr; /* the last gather: the chunk's text, its pairs, the arena bytes it could use */
     uint64_t n = 0, arena_used = 0;
-    void release() { flag.release(); slot.release(); bytes.release(); off.release(); tmp.release(); total.release(); pairs.release(); text.release(); }
+    void release() {
+        mask.release(); has.release(); slot.release(); bytes.release(); off.release(); tmp.release(); total.release();
+        pairs.release(); pair_mask.release(); text.release();
+    }
 };
-/* gf_map_fastq_text's optional output: the lines of every pair that has a record, in ascending pair order (pair_idx counts
- * from the start of the call's text, text_off into `text`) */
+/* gf_map_fastq_text's optional output, per index: the lines of every pair that has a record of that index, in ascending pair
+ * order (pair_idx counts from the start of the call's text, text_off into `text`) */
 struct GfFastqReads {
     std::vector<gf_fastq_read_pair> pairs;
     std::vector<uint8_t> text;
+};
+/* indices one FASTQ stream maps against (one bit each in the per-pair masks of gf_fastq_gather_reads) */
+constexpr uint32_t GF_FASTQ_LIST_MAX = 64;
+/* the final record lists of a list's indices, as kernel parameters (device pointers; the counts are read on the device) */
+struct GfRecordLists {
+    const gf_match* rec[GF_FASTQ_LIST_MAX];
+    const unsigned long long* n[GF_FASTQ_LIST_MAX];
 };
 
 struct GfChunkEvents { /* start, after k_prep, k_seed, k_diag, the whole screen, exact + verify */
@@ -211,22 +222,32 @@ uint32_t gf_scan_launches(uint64_t n); /* kernels gf_exclusive_scan_u32 launches
 
 /* final_chunk: the text ends the file (an unterminated last line is a line); otherwise it is ignored (streamed chunks) */
 int gf_fastq_parse_device(const uint8_t* d_text, uint64_t bytes, GfFastqTable* out, cudaStream_t st, bool final_chunk = true);
-/* gf_api.cu: gf_map_fastq's body.  final_chunk = false (gf_fastq_stream_*): only whole records are mapped and consumed[k]
- * returns how many bytes of buffer k they covered (the caller carries the rest over); pair_idx counts from 0. */
-int gf_map_fastq_text(gf_index* idx, const uint8_t* fq1, uint64_t bytes1, const uint8_t* fq2, uint64_t bytes2, bool final_chunk,
-                      gf_match* out, uint64_t out_cap, uint64_t* n_out, uint64_t* n_records, uint64_t consumed[2],
+/* gf_api.cu: gf_map_fastq's body, against the nh indices hs[] (all on one device, validated by the caller; all of them are
+ * locked for the call).  The text is copied, inflated, split into records and converted once, in hs[0]'s workspace; every
+ * index then screens and verifies it into its own record buffers.  out[h] / out_cap[h] / n_out[h] belong to hs[h]
+ * (GF_E_CAPACITY when any out_cap[h] is too small: n_out[] holds the required counts, nothing is copied).  final_chunk = false
+ * (gf_fastq_stream_*): only whole records are mapped and consumed[k] returns how many bytes of buffer k they covered (the caller
+ * carries the rest over); pair_idx counts from 0.  GF_E_REF_PANIC when any index's records carry the reference's panic; then
+ * panic[h] (when given) says which. */
+int gf_map_fastq_text(gf_index* const* hs, uint32_t nh, const uint8_t* fq1, uint64_t bytes1, const uint8_t* fq2, uint64_t bytes2,
+                      bool final_chunk, gf_match* const* out, const uint64_t* out_cap, uint64_t* n_out, uint64_t* n_records,
+                      uint64_t consumed[2],
                       const GfFastqMembers* members = nullptr /* [2]: BGZF members that follow the host text, inflated on the device */,
-                      GfFastqReads* reads = nullptr /* the lines of the pairs that have a record (nullptr: nothing is gathered) */);
-/* after the records of a FASTQ chunk are final (d_rec[0 .. *d_n_rec), local pair indices): gather the lines of every pair that
- * has one from the chunk's text (text[1] = nullptr: single end) into idx->fq_reads, and queue the copies of the totals into h
+                      GfFastqReads* reads = nullptr /* [nh]: the lines of the pairs that have a record (nullptr: nothing is gathered) */,
+                      bool* panic = nullptr /* [nh] */,
+                      std::vector<uint8_t>* tail = nullptr /* [2]: a mate with members gets its unconsumed text back here (the text
+                                                               exists on the device only; copied while the indices are locked) */);
+/* after the records of a FASTQ chunk are final (lists.rec[h][0 .. *lists.n[h]) for the nh indices of the list, local pair
+ * indices): gather the lines of every pair that has a record of any of them from the chunk's text (text[1] = nullptr: single
+ * end) into idx->fq_reads, with the mask of the indices it belongs to, and queue the copies of the totals into h
  * (n_read_pairs, read_bytes, read_bytes64).  n = records (pairs) of the chunk.  The lines are copied only when they fit the
  * arena as it is: once the totals have arrived, gf_fastq_regather_reads(idx, h->read_bytes64, st) grows it and copies them
  * when they did not (and returns at once when they did); the text and newline tables must still be resident. */
-int gf_fastq_gather_reads(gf_index* idx, const uint8_t* const text[2], uint64_t n, const gf_match* d_rec,
-                          const unsigned long long* d_n_rec, GfHostSlot* h, cudaStream_t st);
+int gf_fastq_gather_reads(gf_index* idx, const uint8_t* const text[2], uint64_t n, const GfRecordLists& lists, uint32_t nh,
+                          GfHostSlot* h, cudaStream_t st);
 int gf_fastq_regather_reads(gf_index* idx, uint64_t bytes, cudaStream_t st);
-/* after gf_map_fastq_text: bytes [from, from + len) of mate k's text as the device saw it (the unconsumed tail of a chunk) */
-int gf_fastq_fetch_text(gf_index* idx, int k, uint64_t from, uint64_t len, uint8_t* dst);
+/* gf_api.cu: the checks of gf_list_map_pairs on a list of handles (non-empty, no NULL, none twice, one device) */
+int gf_validate_list(gf_index* const* hs, uint32_t nh);
 
 /* gf_map.cu */
 struct GfDevBatch {

@@ -24,6 +24,7 @@
 #include <chrono>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <thread>
 #include <vector>
 
@@ -220,8 +221,18 @@ int gf_stream_get_counts(const gf_stream* s, uint64_t* pairs_pushed, uint64_t* m
 } /* extern "C" */
 
 /* ================================================================================================== FASTQ text */
+/* what one index of a FASTQ stream has mapped and not yet taken */
+struct FqIndexOut {
+    std::vector<gf_match> done, tmp;
+    bool panic = false;
+    std::vector<gf_fastq_read_pair> reads; /* ascending pair_idx, text_off into read_text */
+    std::vector<uint8_t> read_text;
+};
+
 struct gf_fastq_stream {
-    gf_index* idx = nullptr;
+    std::vector<gf_index*> idx; /* idx[0]'s workspace holds the text, the newline tables and the sequence store */
+    std::vector<FqIndexOut> per; /* one per index */
+    std::vector<GfFastqReads> chunk_reads; /* per index: what the last mapping call gathered (keep_reads) */
     bool paired = true;
     int format = GF_FQ_PLAIN;
     uint64_t chunk_bytes = 256ull << 20;
@@ -239,14 +250,9 @@ struct gf_fastq_stream {
     uint64_t records = 0, text_bytes = 0, n_calls = 0;
     uint64_t bgzf_blocks = 0; /* members inflated on the parallel path */
     double ms_bgzf = 0, ms_stream = 0, ms_map = 0; /* GF_DEBUG_TIMING: where the host time of the gzip path goes (mate 1's thread) */
-    std::vector<gf_match> done, tmp;
-    bool panic = false;
     bool fed = false;
-    bool keep_reads = false;             /* gf_fastq_stream_keep_reads: the lines of the pairs behind `done` */
-    std::vector<gf_fastq_read_pair> reads; /* ascending pair_idx, text_off into read_text */
-    std::vector<uint8_t> read_text;
-    GfFastqReads chunk_reads;            /* what the last mapping call gathered */
-    std::mutex mu;
+    bool keep_reads = false; /* gf_fastq_stream_keep_reads: the lines of the pairs behind each index's `done` */
+    std::mutex mu;           /* taken before the indices' own locks */
     ~gf_fastq_stream() {
         for (int k = 0; k < 2; k++)
             if (z_open[k]) inflateEnd(&z[k]);
@@ -255,13 +261,18 @@ struct gf_fastq_stream {
 
 namespace {
 
-/* maps the whole records buffered so far; final_chunk: the files have ended */
+/* maps the whole records buffered so far against every index; final_chunk: the files have ended */
 int fq_map_locked(gf_fastq_stream* s, bool final_chunk) {
     const int nm = s->paired ? 2 : 1;
+    const uint32_t nh = (uint32_t)s->idx.size();
     const uint64_t total[2] = {s->text[0].fill + s->pending_text[0], s->text[1].fill + s->pending_text[1]};
     if (total[0] == 0 && (!s->paired || total[1] == 0)) return GF_OK;
-    if (s->tmp.size() < 4096) s->tmp.resize(4096);
-    uint64_t got = 0, nrec = 0, consumed[2] = {0, 0};
+    std::vector<gf_match*> outs(nh);
+    std::vector<uint64_t> caps(nh), got(nh, 0);
+    s->chunk_reads.resize(nh);
+    std::unique_ptr<bool[]> panic(new bool[nh]);
+    uint64_t nrec = 0, consumed[2] = {0, 0};
+    std::vector<uint8_t> tail[2];
     int rc;
     const auto tm0 = std::chrono::steady_clock::now();
     GfFastqMembers mem[2];
@@ -273,29 +284,38 @@ int fq_map_locked(gf_fastq_stream* s, bool final_chunk) {
         mem[k].n_members = (uint32_t)s->members[k].size();
         mem[k].text_bytes = s->pending_text[k];
     }
+    for (uint32_t h = 0; h < nh; h++)
+        if (s->per[h].tmp.size() < 4096) s->per[h].tmp.resize(4096);
     for (;;) {
-        rc = gf_map_fastq_text(s->idx, s->text[0].p, s->text[0].fill, s->paired ? s->text[1].p : nullptr,
-                               s->paired ? s->text[1].fill : 0, final_chunk, s->tmp.data(), s->tmp.size(), &got, &nrec, consumed,
-                               have_members ? mem : nullptr, s->keep_reads ? &s->chunk_reads : nullptr);
-        if (rc == GF_E_CAPACITY) { s->tmp.resize(got); continue; }
+        for (uint32_t h = 0; h < nh; h++) { outs[h] = s->per[h].tmp.data(); caps[h] = s->per[h].tmp.size(); }
+        rc = gf_map_fastq_text(s->idx.data(), nh, s->text[0].p, s->text[0].fill, s->paired ? s->text[1].p : nullptr,
+                               s->paired ? s->text[1].fill : 0, final_chunk, outs.data(), caps.data(), got.data(), &nrec, consumed,
+                               have_members ? mem : nullptr, s->keep_reads ? s->chunk_reads.data() : nullptr, panic.get(), tail);
+        if (rc == GF_E_CAPACITY) {
+            for (uint32_t h = 0; h < nh; h++) s->per[h].tmp.resize(std::max<uint64_t>(got[h], s->per[h].tmp.size()));
+            continue;
+        }
         break;
     }
     s->ms_map += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tm0).count();
     if (rc != GF_OK && rc != GF_E_REF_PANIC) return rc;
-    if (rc == GF_E_REF_PANIC) s->panic = true;
-    for (uint64_t i = 0; i < got; i++) {
-        gf_match m = s->tmp[i];
-        m.pair_idx += s->records;
-        s->done.push_back(m);
-    }
-    if (s->keep_reads) { /* pair numbers and text offsets of the chunk -> the stream's */
-        const uint64_t base = s->read_text.size();
-        for (gf_fastq_read_pair p : s->chunk_reads.pairs) {
-            p.pair_idx += s->records;
-            p.text_off += base;
-            s->reads.push_back(p);
+    for (uint32_t h = 0; h < nh; h++) {
+        FqIndexOut& o = s->per[h];
+        if (panic[h]) o.panic = true;
+        for (uint64_t i = 0; i < got[h]; i++) {
+            gf_match m = o.tmp[i];
+            m.pair_idx += s->records;
+            o.done.push_back(m);
         }
-        s->read_text.insert(s->read_text.end(), s->chunk_reads.text.begin(), s->chunk_reads.text.end());
+        if (s->keep_reads) { /* pair numbers and text offsets of the chunk -> the stream's */
+            const uint64_t base = o.read_text.size();
+            for (gf_fastq_read_pair p : s->chunk_reads[h].pairs) {
+                p.pair_idx += s->records;
+                p.text_off += base;
+                o.reads.push_back(p);
+            }
+            o.read_text.insert(o.read_text.end(), s->chunk_reads[h].text.begin(), s->chunk_reads[h].text.end());
+        }
     }
     s->records += nrec;
     s->n_calls++;
@@ -309,12 +329,10 @@ int fq_map_locked(gf_fastq_stream* s, bool final_chunk) {
             memmove(t.p, t.p + c, t.fill - c);
             t.fill -= c;
         } else {
-            /* the unconsumed tail (usually the last, incomplete record) comes back from the device and opens the next chunk */
-            const uint64_t tail = total[k] - c;
-            if (t.reserve(tail + 64) != cudaSuccess) return sfail(GF_E_CUDA, "pinned allocation failed");
-            int r = gf_fastq_fetch_text(s->idx, k, c, tail, t.p);
-            if (r != GF_OK) return r;
-            t.fill = tail;
+            /* the unconsumed tail (usually the last, incomplete record) came back from the device and opens the next chunk */
+            if (t.reserve(tail[k].size() + 64) != cudaSuccess) return sfail(GF_E_CUDA, "pinned allocation failed");
+            if (!tail[k].empty()) memcpy(t.p, tail[k].data(), tail[k].size());
+            t.fill = tail[k].size();
         }
         s->members[k].clear();
         s->comp[k].fill = 0;
@@ -585,17 +603,27 @@ int fq_append(gf_fastq_stream* s, int k, const uint8_t* in, uint64_t n, uint64_t
 
 extern "C" {
 
-int gf_fastq_stream_create(gf_index* idx, int paired, int format, uint64_t chunk_bytes, gf_fastq_stream** out) {
-    if (!idx || !out) return sfail(GF_E_INVALID, "NULL argument");
+int gf_fastq_stream_create_list(gf_index* const* idx, uint32_t n_idx, int paired, int format, uint64_t chunk_bytes,
+                                gf_fastq_stream** out) {
+    if (!out) return sfail(GF_E_INVALID, "NULL argument");
+    int rc = gf_validate_list(idx, n_idx);
+    if (rc != GF_OK) return rc;
+    if (n_idx > GF_FASTQ_LIST_MAX) return sfail(GF_E_LIMIT, "a FASTQ stream maps against at most 64 indices");
     if (format != GF_FQ_PLAIN && format != GF_FQ_GZIP) return sfail(GF_E_INVALID, "unknown FASTQ format");
     gf_fastq_stream* s = new gf_fastq_stream();
-    s->idx = idx;
+    s->idx.assign(idx, idx + n_idx);
+    s->per.resize(n_idx);
     s->paired = paired != 0;
     s->format = format;
     if (chunk_bytes) s->chunk_bytes = std::max<uint64_t>(chunk_bytes, 4096);
     { const char* e = getenv("GF_BGZF_DEVICE"); s->device_inflate = !(e && atoi(e) == 0); }
     *out = s;
     return GF_OK;
+}
+
+int gf_fastq_stream_create(gf_index* idx, int paired, int format, uint64_t chunk_bytes, gf_fastq_stream** out) {
+    if (!idx) return sfail(GF_E_INVALID, "NULL argument");
+    return gf_fastq_stream_create_list(&idx, 1, paired, format, chunk_bytes, out);
 }
 
 void gf_fastq_stream_destroy(gf_fastq_stream* s) {
@@ -611,7 +639,7 @@ int gf_fastq_stream_feed(gf_fastq_stream* s, const uint8_t* fq1, uint64_t n1, co
     if (!s || (n1 && !fq1) || (n2 && !fq2)) return sfail(GF_E_INVALID, "NULL argument");
     if (!s->paired && n2) return sfail(GF_E_INVALID, "single-end stream fed with a second file");
     std::lock_guard<std::mutex> lk(s->mu);
-    GF_CUDA_TRY(cudaSetDevice(s->idx->device));
+    GF_CUDA_TRY(cudaSetDevice(s->idx[0]->device));
     s->fed = true;
     const uint8_t* in[2] = {fq1, fq2};
     uint64_t left[2] = {n1, n2};
@@ -653,7 +681,7 @@ int gf_fastq_stream_feed(gf_fastq_stream* s, const uint8_t* fq1, uint64_t n1, co
 int gf_fastq_stream_finish(gf_fastq_stream* s) {
     if (!s) return sfail(GF_E_INVALID, "NULL argument");
     std::lock_guard<std::mutex> lk(s->mu);
-    GF_CUDA_TRY(cudaSetDevice(s->idx->device));
+    GF_CUDA_TRY(cudaSetDevice(s->idx[0]->device));
     if (s->format == GF_FQ_GZIP)
         for (int k = 0; k < (s->paired ? 2 : 1); k++)
             if ((s->z_open[k] && !s->z_member_done[k]) || !s->carry[k].empty())
@@ -661,21 +689,28 @@ int gf_fastq_stream_finish(gf_fastq_stream* s) {
     return fq_map_locked(s, true);
 }
 
-int gf_fastq_stream_take(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out) {
+int gf_fastq_stream_take_index(gf_fastq_stream* s, uint32_t index, gf_match* out, uint64_t out_cap, uint64_t* n_out) {
     if (!s || !n_out) return sfail(GF_E_INVALID, "NULL argument");
     std::lock_guard<std::mutex> lk(s->mu);
+    if (index >= s->idx.size()) return sfail(GF_E_INVALID, "index out of range");
     if (s->keep_reads) return sfail(GF_E_INVALID, "the stream keeps reads: collect records with gf_fastq_stream_take_reads");
-    *n_out = s->done.size();
-    if (s->done.size() > out_cap) return sfail(GF_E_CAPACITY, "out_cap too small; *n_out holds the required count");
-    if (!out && !s->done.empty()) return sfail(GF_E_INVALID, "out is NULL");
-    sort_records(s->idx, s->done);
-    if (!s->done.empty()) memcpy(out, s->done.data(), sizeof(gf_match) * s->done.size());
-    s->done.clear();
-    if (s->panic) {
-        s->panic = false;
+    FqIndexOut& o = s->per[index];
+    *n_out = o.done.size();
+    if (o.done.size() > out_cap) return sfail(GF_E_CAPACITY, "out_cap too small; *n_out holds the required count");
+    if (!out && !o.done.empty()) return sfail(GF_E_INVALID, "out is NULL");
+    sort_records(s->idx[index], o.done);
+    if (!o.done.empty()) memcpy(out, o.done.data(), sizeof(gf_match) * o.done.size());
+    o.done.clear();
+    if (o.panic) {
+        o.panic = false;
         return sfail(GF_E_REF_PANIC, "a candidate needs an edit distance over more than 640 columns (reference panics)");
     }
     return GF_OK;
+}
+
+int gf_fastq_stream_take(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out) {
+    if (s && s->idx.size() != 1) return sfail(GF_E_INVALID, "the stream maps against several indices: use gf_fastq_stream_take_index");
+    return gf_fastq_stream_take_index(s, 0, out, out_cap, n_out);
 }
 
 int gf_fastq_stream_keep_reads(gf_fastq_stream* s) {
@@ -686,30 +721,39 @@ int gf_fastq_stream_keep_reads(gf_fastq_stream* s) {
     return GF_OK;
 }
 
-int gf_fastq_stream_take_reads(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out, gf_fastq_read_pair* pairs,
-                               uint64_t pairs_cap, uint64_t* n_pairs, uint8_t* text, uint64_t text_cap, uint64_t* n_text) {
+int gf_fastq_stream_take_reads_index(gf_fastq_stream* s, uint32_t index, gf_match* out, uint64_t out_cap, uint64_t* n_out,
+                                     gf_fastq_read_pair* pairs, uint64_t pairs_cap, uint64_t* n_pairs, uint8_t* text,
+                                     uint64_t text_cap, uint64_t* n_text) {
     if (!s || !n_out || !n_pairs || !n_text) return sfail(GF_E_INVALID, "NULL argument");
     std::lock_guard<std::mutex> lk(s->mu);
+    if (index >= s->idx.size()) return sfail(GF_E_INVALID, "index out of range");
     if (!s->keep_reads) return sfail(GF_E_INVALID, "the stream does not keep reads (gf_fastq_stream_keep_reads)");
-    *n_out = s->done.size();
-    *n_pairs = s->reads.size();
-    *n_text = s->read_text.size();
-    if (s->done.size() > out_cap || s->reads.size() > pairs_cap || s->read_text.size() > text_cap)
+    FqIndexOut& o = s->per[index];
+    *n_out = o.done.size();
+    *n_pairs = o.reads.size();
+    *n_text = o.read_text.size();
+    if (o.done.size() > out_cap || o.reads.size() > pairs_cap || o.read_text.size() > text_cap)
         return sfail(GF_E_CAPACITY, "a capacity is too small; *n_out, *n_pairs and *n_text hold the required counts");
-    if ((!out && !s->done.empty()) || (!pairs && !s->reads.empty()) || (!text && !s->read_text.empty()))
+    if ((!out && !o.done.empty()) || (!pairs && !o.reads.empty()) || (!text && !o.read_text.empty()))
         return sfail(GF_E_INVALID, "output buffer is NULL");
-    sort_records(s->idx, s->done);
-    if (!s->done.empty()) memcpy(out, s->done.data(), sizeof(gf_match) * s->done.size());
-    if (!s->reads.empty()) memcpy(pairs, s->reads.data(), sizeof(gf_fastq_read_pair) * s->reads.size());
-    if (!s->read_text.empty()) memcpy(text, s->read_text.data(), s->read_text.size());
-    s->done.clear();
-    s->reads.clear();
-    s->read_text.clear();
-    if (s->panic) {
-        s->panic = false;
+    sort_records(s->idx[index], o.done);
+    if (!o.done.empty()) memcpy(out, o.done.data(), sizeof(gf_match) * o.done.size());
+    if (!o.reads.empty()) memcpy(pairs, o.reads.data(), sizeof(gf_fastq_read_pair) * o.reads.size());
+    if (!o.read_text.empty()) memcpy(text, o.read_text.data(), o.read_text.size());
+    o.done.clear();
+    o.reads.clear();
+    o.read_text.clear();
+    if (o.panic) {
+        o.panic = false;
         return sfail(GF_E_REF_PANIC, "a candidate needs an edit distance over more than 640 columns (reference panics)");
     }
     return GF_OK;
+}
+
+int gf_fastq_stream_take_reads(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out, gf_fastq_read_pair* pairs,
+                               uint64_t pairs_cap, uint64_t* n_pairs, uint8_t* text, uint64_t text_cap, uint64_t* n_text) {
+    if (s && s->idx.size() != 1) return sfail(GF_E_INVALID, "the stream maps against several indices: use gf_fastq_stream_take_reads_index");
+    return gf_fastq_stream_take_reads_index(s, 0, out, out_cap, n_out, pairs, pairs_cap, n_pairs, text, text_cap, n_text);
 }
 
 int gf_fastq_stream_get_counts(const gf_fastq_stream* s, uint64_t* records, uint64_t* text_bytes, uint64_t* map_calls) {

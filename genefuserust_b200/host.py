@@ -459,10 +459,15 @@ class FastqStream:
     anywhere), whole records are split and mapped on the device; records are numbered from the start of the files."""
 
     def __init__(self, mapper, paired=True, gz=False, chunk_bytes=0, keep_reads=False):
-        """keep_reads: gather the FASTQ lines of every pair that has a record on the device (collect them with take_reads)"""
-        self.lib = mapper.lib
+        """mapper: one FusionMapper, or a list of them (list mode: every chunk is inflated, split and converted once and mapped
+        against each; collect mapper k's records with take(k) / take_reads(k)).
+        keep_reads: gather the FASTQ lines of every pair that has a record on the device (collect them with take_reads)"""
+        mappers = list(mapper) if isinstance(mapper, (list, tuple)) else [mapper]
+        self.lib = mappers[0].lib
         h = C.c_void_p()
-        _check(self.lib, self.lib.gf_fastq_stream_create(mapper.m_indexer.h, 1 if paired else 0, 1 if gz else 0, chunk_bytes, C.byref(h)))
+        handles = (C.c_void_p * len(mappers))(*[m.m_indexer.h for m in mappers])
+        _check(self.lib, self.lib.gf_fastq_stream_create_list(handles, len(mappers), 1 if paired else 0, 1 if gz else 0, chunk_bytes,
+                                                              C.byref(h)))
         self.h = h
         self.paired = paired
         if keep_reads:
@@ -474,29 +479,30 @@ class FastqStream:
     def finish(self):
         _check(self.lib, self.lib.gf_fastq_stream_finish(self.h))
 
-    def take(self):
+    def take(self, index=0):
+        """the records of mapper `index` (of the list the stream was made with) mapped since its last take"""
         cap = 4096
         while True:
             out = (gf_match * cap)()
             n = C.c_uint64(0)
-            rc = self.lib.gf_fastq_stream_take(self.h, out, cap, C.byref(n))
+            rc = self.lib.gf_fastq_stream_take_index(self.h, index, out, cap, C.byref(n))
             if rc == GF_E_CAPACITY:
                 cap = int(n.value)
                 continue
             _check(self.lib, rc, allow=(GF_E_REF_PANIC,))
             return [out[i] for i in range(n.value)]
 
-    def take_reads(self):
-        """(records, {pair_idx: ((name, seq, strand, qual) of mate 1, the same of mate 2 or None)}) of a stream that keeps
-        reads: the lines exactly as FastqReader::read yields them"""
+    def take_reads(self, index=0):
+        """(records, {pair_idx: ((name, seq, strand, qual) of mate 1, the same of mate 2 or None)}) of mapper `index` on a
+        stream that keeps reads: the lines exactly as FastqReader::read yields them, of that mapper's records' pairs"""
         caps = [4096, 4096, 1 << 20]
         while True:
             out = (gf_match * caps[0])()
             pairs = (gf_fastq_read_pair * caps[1])()
             text = (C.c_uint8 * caps[2])()
             n, npair, ntext = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
-            rc = self.lib.gf_fastq_stream_take_reads(self.h, out, caps[0], C.byref(n), pairs, caps[1], C.byref(npair),
-                                                     text, caps[2], C.byref(ntext))
+            rc = self.lib.gf_fastq_stream_take_reads_index(self.h, index, out, caps[0], C.byref(n), pairs, caps[1], C.byref(npair),
+                                                           text, caps[2], C.byref(ntext))
             if rc == GF_E_CAPACITY:
                 caps = [max(caps[0], int(n.value)), max(caps[1], int(npair.value)), max(caps[2], int(ntext.value))]
                 continue

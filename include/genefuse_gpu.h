@@ -422,6 +422,29 @@ int gf_fastq_stream_keep_reads(gf_fastq_stream* s);
 int gf_fastq_stream_take_reads(gf_fastq_stream* s, gf_match* out, uint64_t out_cap, uint64_t* n_out,
                                gf_fastq_read_pair* pairs, uint64_t pairs_cap, uint64_t* n_pairs,
                                uint8_t* text, uint64_t text_cap, uint64_t* n_text);
+/* One stream, several fusion CSVs (list mode on FASTQ input, src/core/fusion_scan.rs:62-188).  gf_fastq_stream_create_list
+ * maps every chunk against the n_idx indices idx[]: the chunk is copied, inflated, split into records and converted ONCE, then
+ * screened and verified per index.  The list is checked like gf_list_map_pairs checks it: non-empty, no NULL, no handle twice,
+ * all handles on one device (GF_E_INVALID otherwise); more than 64 handles gives GF_E_LIMIT.  gf_fastq_stream_create(idx, ...)
+ * is the list of one.  feed, finish, keep_reads and get_counts are unchanged; records are numbered from the start of the files,
+ * the same for every index.
+ * gf_fastq_stream_take_index(s, h, ...) returns exactly what gf_fastq_stream_take returns on a stream over idx[h] alone, fed the
+ * same pieces with takes at the same points: the same records in the same order (idx[h]'s own output mode, bucket order when
+ * idx[h] has it set), the same GF_E_CAPACITY protocol and the GF_E_REF_PANIC rule per index (only an index whose own records
+ * carry the panic reports it).  gf_fastq_stream_take_reads_index is the same for gf_fastq_stream_take_reads: its records,
+ * descriptors (text_off included) and text are byte-identical to the single-index stream's, so index h gets the pairs of its
+ * own records only.  A take consumes only that index's records and lines.  On a stream with more than one index
+ * gf_fastq_stream_take / take_reads fail with GF_E_INVALID; so does an index >= n_idx.
+ * The handles must outlive the stream.  While a chunk is mapped all of them are locked (in address order, like
+ * gf_list_map_pairs), after the stream's own lock.  Device memory: the chunk's text, its newline tables, the sequence store
+ * and the gathered lines live in idx[0]'s workspace; every handle keeps its own record buffers for a chunk (up to 2 records
+ * per pair: 48 B each, twice with an output mode, plus 8 B of sort key per record with one). */
+int gf_fastq_stream_create_list(gf_index* const* idx, uint32_t n_idx, int paired, int format, uint64_t chunk_bytes,
+                                gf_fastq_stream** out);
+int gf_fastq_stream_take_index(gf_fastq_stream* s, uint32_t index, gf_match* out, uint64_t out_cap, uint64_t* n_out);
+int gf_fastq_stream_take_reads_index(gf_fastq_stream* s, uint32_t index, gf_match* out, uint64_t out_cap, uint64_t* n_out,
+                                     gf_fastq_read_pair* pairs, uint64_t pairs_cap, uint64_t* n_pairs,
+                                     uint8_t* text, uint64_t text_cap, uint64_t* n_text);
 
 /* ---- the packed upload, as a host-side utility ----
  * With all four arenas of a batch in pinned host memory (and reads <= 256 bases) gf_map_pairs / gf_list_map_pairs do not copy

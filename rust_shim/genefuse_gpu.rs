@@ -73,6 +73,12 @@ extern "C" {
     fn gf_fastq_stream_take_reads(s: *mut gf_fastq_stream, out: *mut gf_match, out_cap: u64, n_out: *mut u64,
                                   pairs: *mut gf_fastq_read_pair, pairs_cap: u64, n_pairs: *mut u64,
                                   text: *mut u8, text_cap: u64, n_text: *mut u64) -> c_int;
+    fn gf_fastq_stream_create_list(idx: *const *mut gf_index, n_idx: u32, paired: c_int, format: c_int, chunk_bytes: u64,
+                                   out: *mut *mut gf_fastq_stream) -> c_int;
+    fn gf_fastq_stream_take_index(s: *mut gf_fastq_stream, index: u32, out: *mut gf_match, out_cap: u64, n_out: *mut u64) -> c_int;
+    fn gf_fastq_stream_take_reads_index(s: *mut gf_fastq_stream, index: u32, out: *mut gf_match, out_cap: u64, n_out: *mut u64,
+                                        pairs: *mut gf_fastq_read_pair, pairs_cap: u64, n_pairs: *mut u64,
+                                        text: *mut u8, text_cap: u64, n_text: *mut u64) -> c_int;
     fn gf_reference_create(contigs: *const gf_ref_contig, n_contigs: u32, device: c_int, out: *mut *mut gf_reference) -> c_int;
     fn gf_reference_destroy(r: *mut gf_reference);
     fn gf_alignable_filter(r: *mut gf_reference, seqs: *const u8, seq_off: *const u64, n_seqs: u64, alignable: *mut u8,
@@ -223,6 +229,9 @@ impl Drop for PackStream { fn drop(&mut self) { unsafe { gf_stream_destroy(self.
 /// they are read (`.fq` plain, `.fq.gz` with gzip = true: BGZF members are inflated on the device); whole records are split and
 /// mapped on the device.  With keep_reads the stream also returns the four lines of both mates of every matched pair, which is
 /// all a ReadMatch needs (take_reads); without it, take() returns the records alone.
+/// List mode (src/core/fusion_scan.rs:62-188 on FASTQ input): new_list maps every chunk against several indices — the chunk is
+/// inflated, split and converted once — and take_index(h) / take_reads_index(h) return exactly what a stream over indices[h]
+/// alone would.  The indices must outlive the stream.
 pub struct FastqStream { s: *mut gf_fastq_stream, paired: bool }
 unsafe impl Send for FastqStream {}
 unsafe impl Sync for FastqStream {} // calls on one stream are serialised inside the library
@@ -253,9 +262,16 @@ impl FastqReads {
 impl FastqStream {
     /// chunk_bytes = 0: 256 MiB of text per mate per mapping call
     pub fn new(index: &GpuIndex, paired: bool, gzip: bool, chunk_bytes: u64, keep_reads: bool) -> Result<Self, String> {
+        Self::new_list(&[index], paired, gzip, chunk_bytes, keep_reads)
+    }
+    /// one stream against several indices (at most 64, all on one device, none twice)
+    pub fn new_list(indices: &[&GpuIndex], paired: bool, gzip: bool, chunk_bytes: u64, keep_reads: bool) -> Result<Self, String> {
+        let hs: Vec<*mut gf_index> = indices.iter().map(|g| g.h).collect();
         let mut s: *mut gf_fastq_stream = std::ptr::null_mut();
         let fmt = if gzip { GF_FQ_GZIP } else { GF_FQ_PLAIN };
-        if unsafe { gf_fastq_stream_create(index.h, paired as c_int, fmt, chunk_bytes, &mut s) } != 0 { return Err(last_error()); }
+        if unsafe { gf_fastq_stream_create_list(hs.as_ptr(), hs.len() as u32, paired as c_int, fmt, chunk_bytes, &mut s) } != 0 {
+            return Err(last_error());
+        }
         let st = Self { s, paired };
         if keep_reads && unsafe { gf_fastq_stream_keep_reads(st.s) } != 0 { return Err(last_error()); }
         Ok(st)
@@ -266,28 +282,33 @@ impl FastqStream {
     }
     /// end of the files: the last records are mapped
     pub fn finish(&self) -> Result<(), String> { if unsafe { gf_fastq_stream_finish(self.s) } != 0 { Err(last_error()) } else { Ok(()) } }
-    pub fn take(&self) -> Result<Vec<gf_match>, String> {
+    /// the records of a one-index stream (take_index(0))
+    pub fn take(&self) -> Result<Vec<gf_match>, String> { self.take_index(0) }
+    /// the records of indices[index] mapped since its last take
+    pub fn take_index(&self, index: u32) -> Result<Vec<gf_match>, String> {
         let mut cap = 4096usize;
         loop {
             let mut out = vec![gf_match::default(); cap];
             let mut n = 0u64;
-            let rc = unsafe { gf_fastq_stream_take(self.s, out.as_mut_ptr(), cap as u64, &mut n) };
+            let rc = unsafe { gf_fastq_stream_take_index(self.s, index, out.as_mut_ptr(), cap as u64, &mut n) };
             if rc == GF_E_CAPACITY { cap = n as usize; continue; }
             if rc != 0 { return Err(last_error()); }
             out.truncate(n as usize);
             return Ok(out);
         }
     }
-    /// the records (as take() would return them) and the lines of every pair among them
-    pub fn take_reads(&self) -> Result<FastqReads, String> {
+    /// the records (as take() would return them) and the lines of every pair among them, of a one-index stream
+    pub fn take_reads(&self) -> Result<FastqReads, String> { self.take_reads_index(0) }
+    /// take_reads for indices[index]: its records and the lines of its records' pairs only
+    pub fn take_reads_index(&self, index: u32) -> Result<FastqReads, String> {
         let mut caps = [4096u64, 4096, 1 << 20];
         loop {
             let mut out = vec![gf_match::default(); caps[0] as usize];
             let mut pairs = vec![gf_fastq_read_pair::default(); caps[1] as usize];
             let mut text = vec![0u8; caps[2] as usize];
             let mut n = [0u64; 3];
-            let rc = unsafe { gf_fastq_stream_take_reads(self.s, out.as_mut_ptr(), caps[0], &mut n[0], pairs.as_mut_ptr(), caps[1],
-                                                         &mut n[1], text.as_mut_ptr(), caps[2], &mut n[2]) };
+            let rc = unsafe { gf_fastq_stream_take_reads_index(self.s, index, out.as_mut_ptr(), caps[0], &mut n[0], pairs.as_mut_ptr(),
+                                                               caps[1], &mut n[1], text.as_mut_ptr(), caps[2], &mut n[2]) };
             if rc == GF_E_CAPACITY { for k in 0..3 { caps[k] = caps[k].max(n[k]); } continue; }
             if rc != 0 { return Err(last_error()); } // GF_E_REF_PANIC included: the reference aborts there
             out.truncate(n[0] as usize);
